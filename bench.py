@@ -21,6 +21,7 @@ un-vendored crates and cannot be built in this image) on all host cores: the lin
 (same config as the GPU arm) and the faithful-cost port (quadratic) on a bounded sample.
 """
 import argparse
+import hashlib
 import json
 import os
 import subprocess
@@ -122,6 +123,49 @@ def build_bytes(n_tuples, n_unique):
 def search_bytes(q_res, q_hashes, hits, pairs):
     """SURVEY 8(d): query in, one key probe + row_ptr pair per query hash, postings + hit rows, 48 B of scores per pair."""
     return q_res + q_hashes * 8 + q_hashes * 16 + hits * 8 + hits * 20 + pairs * 48
+
+
+# --dump-outputs: rows kept per column.  The dumped tables have at most 43 float64 columns of this length (index and
+# target index: hash hi/lo, row start hi/lo, row length hi/lo, posting pid, pos; search: 6 hit and 21 pair columns),
+# about 43 MB in all.
+DUMP_ROWS = 1 << 17
+DUMP_SEED = 20260101
+
+
+def dump_columns(prefix, cols):
+    """One result table (columns of equal length) as {prefix + column: float64 array}: every row when there are at most
+    DUMP_ROWS, else the same seeded sample of rows in every column.  A 64-bit integer column becomes its exact 32-bit
+    halves `<column>_hi` / `<column>_lo`; every integer column also gets `<column>_sha256`, the digest of the whole
+    column as eight 32-bit words, so that the rows outside the sample are compared too."""
+    n = len(next(iter(cols.values())))
+    rows = None if n <= DUMP_ROWS else np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_ROWS, replace=False))
+    out = {}
+    for name, a in cols.items():
+        a = np.ascontiguousarray(a)
+        s = a if rows is None else a[rows]
+        if a.dtype.kind in "ui":
+            out[prefix + name + "_sha256"] = np.frombuffer(hashlib.sha256(a).digest(), dtype="<u4").astype(np.float64)
+            if a.dtype.itemsize == 8:
+                s = s.astype(np.uint64)
+                out[prefix + name + "_hi"] = (s >> np.uint64(32)).astype(np.float64)
+                out[prefix + name + "_lo"] = (s & np.uint64(0xFFFFFFFF)).astype(np.float64)
+                continue
+        out[prefix + name] = s.astype(np.float64)
+    return out
+
+
+def dump_index(prefix, idx):
+    """The finalized index as a caller of ks_index_csr receives it: sorted unique hashes with their posting rows, and
+    the postings (protein, position)."""
+    keys, row_ptr, pid, pos = idx.csr()
+    return {**dump_columns(prefix + "key_", {"hash": keys, "row_start": row_ptr[:-1], "row_len": np.diff(row_ptr)}),
+            **dump_columns(prefix + "posting_", {"pid": pid, "pos": pos})}
+
+
+def write_dump(directory, arrays):
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 _PROTEOME_CACHE = {}
@@ -241,7 +285,16 @@ def main():
     ap.add_argument("--cpu-fast-sample", type=int, default=20_000_000)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="skip the target-run and ingest legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps of each leg, write what its last timed step returned (rank 0's index, "
+                         "the search leg's pairs and hits, the target run's index) as DIR/<name>.npy in float64: every "
+                         "row of a small table, a fixed seeded sample of a large one, and a SHA-256 of every whole "
+                         "integer column; the inputs are seeded, so two builds can be compared file by file")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.workload == "c5_sweep" or args.impl == "reference"):
+        ap.error("--dump-outputs applies to the GPU index build workloads")
     if args.workload == "c5_sweep":
         return run_c5_sweep(args)
     cfg = WORKLOADS[args.workload]
@@ -372,6 +425,9 @@ def main():
     e2e_value = total_res / (ms_e2e * 1e-3)
     clocks = sampler.stop() if rank == 0 else None
     st = b.idx.stats()
+    dump = {}
+    if args.dump_outputs and rank == 0:
+        dump.update(dump_index("index_", b.idx))
     n_tuples, n_unique, n_groups = sum_over_ranks(st["n_tuples"], st["n_unique_hashes"], st["n_groups"])
     n_prot_total = sum_over_ranks(len(offs) - 1)[0] if blockwise else len(offs) - 1
     h2d = sum_over_ranks((b.n_res + 7) // 8 * 5 + 72 + (b.n_prot + 1) * 8)[0]
@@ -380,6 +436,8 @@ def main():
 
     # ---- search leg: BASELINE.json configs[2] -- planted query domains against the same proteome, dayhoff k=16 ----
     if blockwise:
+        if dump:
+            write_dump(args.dump_outputs, dump)
         return finish_build_only(args, cfg, rank, world, comm, dist if world > 1 else None, peaks, value, ms_step, e2e_value, ms_e2e,
                                  total_res, n_prot_total, n_tuples, n_unique, h2d, build_path, stage, launches, clocks, W)
     scfg = WORKLOADS[SEARCH_WORKLOAD] if cfg["n_residues"] == WORKLOADS[SEARCH_WORKLOAD]["n_residues"] else dict(cfg, k=16, moltype="dayhoff", scaled=1)
@@ -415,6 +473,9 @@ def main():
                          "value": q_residues * total_res / (wall_ms * 1e-3)}
         if rank == 0 and label == "pairs":
             keep = {c: out["pairs"][c].copy() for c in ("pair_qid", "pair_pid", "intersect_hashes", "containment")}
+        if args.dump_outputs and rank == 0 and hits:
+            dump.update(dump_columns("search_", dict(out["pairs"].items())))
+            dump.update(dump_columns("search_", dict(out["hits"].items())))
     sb.close()
     verify = None
     if world > 1 and rank == 0:
@@ -444,6 +505,8 @@ def main():
             tb.from_host()
         t_e2e = tb.timed(tb.from_host, args.steps) / args.steps
         tst = tb.idx.stats()
+        if args.dump_outputs and rank == 0:
+            dump.update(dump_index("target_index_", tb.idx))
         tt, tu = sum_over_ranks(tst["n_tuples"], tst["n_unique_hashes"])
         tbytes = sketch_bytes(int(toffs[-1]), len(toffs) - 1, tt) + build_bytes(tt, tu)
         extra["target_100m_dayhoff_k16_s1"] = {
@@ -461,6 +524,8 @@ def main():
         if world > 1:
             dist.destroy_process_group()
         return
+    if dump:
+        write_dump(args.dump_outputs, dump)
 
     # ---- roofline (SURVEY 8(d) bytes; stage times are CUDA events the library records on its own stream) ----
     peak, peak_src = peaks()
