@@ -387,16 +387,6 @@ void ks_proteome_free(ks_proteome* p) { delete p; }
 // ------------------------------------------------------------------------------------------------
 namespace {
 
-struct DeviceBatch {  // residues + offsets resident in HBM
-    uint8_t* res = nullptr;
-    uint64_t* offs = nullptr;
-    uint64_t res_cap = 0, offs_cap = 0;
-    uint64_t n_prot = 0, n_res = 0, n_windows = 0;
-    uint64_t max_len = 0;  // longest protein of the batch
-    bool valid = false;
-    bool packed = false;  // res holds 5-bit codes
-};
-
 // Grow-only device buffer: steady-state steps (clear + build again) never go back to the allocator.
 struct Buf {
     void* p = nullptr;
@@ -413,11 +403,16 @@ struct Buf {
     }
 };
 
-uint64_t max_protein_len(const uint64_t* offs, uint64_t n_prot) {
-    uint64_t m = 0;
-    for (uint64_t i = 0; i < n_prot; i++) m = std::max(m, offs[i + 1] - offs[i]);
-    return m;
-}
+struct DeviceBatch {  // residues + offsets resident in HBM
+    uint8_t* res = nullptr;
+    uint64_t* offs = nullptr;
+    Buf b_res, b_offs;  // (a batch of the handle)
+    uint64_t n_prot = 0, n_res = 0, n_windows = 0;
+    uint64_t max_len = 0;  // longest protein of the batch
+    bool valid = false;
+    bool packed = false;  // res holds 5-bit codes
+    uint64_t res_bytes() const { return packed ? packed_bytes(n_res) : n_res + 64; }
+};
 
 // k-mer windows and longest protein of a proteome for k-mer size k (cached on the proteome: one pass per k)
 void proteome_shape(const ks_proteome* cp, uint32_t k, uint64_t* n_windows, uint64_t* max_len) {
@@ -437,14 +432,45 @@ void proteome_shape(const ks_proteome* cp, uint32_t k, uint64_t* n_windows, uint
     *max_len = p->shape_max_len;
 }
 
-uint64_t count_windows(const uint64_t* offs, uint64_t n_prot, uint32_t k) {
-    uint64_t w = 0;
-    for (uint64_t i = 0; i < n_prot; i++) {
-        uint64_t len = offs[i + 1] - offs[i];
-        if (len >= k) w += len - k + 1;
-    }
-    return w;
-}
+// What a handle holds.  The four values between Tuples and Finalized are a pending batch: the resident batch, added as the
+// handle's only content by a route that finalize completes.  n_tuples / n_prot / n_res / n_windows count it already.
+enum class Build {
+    Tuples,              // (protein, pos)-ordered tuples in d_hash / d_loc [0, n_tuples), possibly none: finalize sorts them
+    DenseDeferred,       // the batch is counted, not sketched: finalize runs the dense path's rank kernel over it, then
+                         // builds from the keys
+    DenseRanked,         // the pipelined add has run the rank kernel: the keys are in the dense work buffer (in d_hash when
+                         // the library sorts them), the kernel's flags in d_status; finalize builds from them
+    Scattered,           // the tuples are in the first-level regions of the unstable partition (b_pair_work, pair_plan) and
+                         // the kernel's count has been checked; scaled > 1: t_abund holds the kept windows per protein.
+                         // finalize runs the second level and the bin kernel, the postings go to d_loc
+    ScatteredUnchecked,  // as Scattered, at scaled == 1: the kernel's count and zero-hash flag (d_count) are read back with
+                         // finalize's results
+    Finalized,           // csr is the index; adds fail until ks_index_clear
+};
+
+// The finalized index: views into the handle's grow-only buffers and, for the segmented layout, into the build's scratch
+// (which stays with the handle until the next build).  Meaningful in state Finalized only.
+struct Csr {
+    uint64_t* keys = nullptr;
+    uint32_t *key_grp = nullptr, *grp_start = nullptr, *t_size = nullptr, *t_abund = nullptr, *dir = nullptr;
+    uint64_t* d_counts = nullptr;
+    int dir_bits = 0, dir_shift = 0;
+    int dir_sub = DIR_SUB_COMPACT;  // layout of keys / key_grp / grp_start (index_build.cuh): compact, or segmented
+    uint32_t seg_nb = 0;
+    const uint32_t* seg_start = nullptr;
+    const uint64_t* seg_counts = nullptr;
+    uint64_t U = 0, G = 0, n_ids = 0;
+    bool hash_col_valid = true;  // false: d_hash of the sorted tuples is rebuilt on demand (ks_index_export)
+};
+
+// The device words a build reports through (ks_index::d_status), one block so that they are zeroed and read back together.
+struct StatusBlock {
+    uint64_t U, G;         // CSR totals (d_counts)
+    uint64_t produced;     // tuples of the sketch kernel (d_count[0])
+    uint64_t zero_flag;    // high word != 0: a zero hash on the exact path (d_count[1])
+    uint64_t dense_flags;  // dense path, u32 pair: unhandled exception | exception keys emitted
+    uint64_t overflow;     // u32: a sort bucket of the dense path overflowed (the unstable partition's own flag is read here)
+};
 
 }  // namespace
 
@@ -487,22 +513,17 @@ struct ks_index {
     Arena* arena = nullptr;
 
     DeviceBatch batch, qbatch;
+    Build state = Build::Tuples;
     // tuples
     uint64_t *d_hash = nullptr, *d_loc = nullptr;
     uint64_t cap = 0, n_tuples = 0;
     uint64_t n_prot = 0, n_res = 0, n_windows = 0;
-    // device words a build reports through, one block so that they are zeroed and read back together:
-    // [0..1] CSR totals (d_counts), [2..3] sketch count + zero-hash flag (d_count), [4] dense path flags (u32 pair:
-    // unhandled exception | exception keys emitted), [5] dense path: a sort bucket overflowed (u32)
-    uint64_t* d_status = nullptr;
-    uint64_t* d_count = nullptr;
+    uint64_t* d_status = nullptr;  // StatusBlock
+    uint64_t* d_count = nullptr;   // d_status + 2
     void* ws = nullptr;
     size_t ws_bytes = 0;
-    // csr
-    bool finalized = false;
-    bool hash_col_valid = true;  // false: d_hash of the sorted tuples is rebuilt on demand (ks_index_export)
     // dense k-mer space path (hp, 8 <= k <= 24, scaled == 1): per-handle rank tables; a batch that qualifies is not
-    // sketched when it is added but built as a whole by finalize (pending_dense)
+    // sketched when it is added but built as a whole by finalize (Build::DenseDeferred)
     int dense_state = 0;  // 0: tables not built, 1: ready, -1: unusable for this k (two patterns share a hash)
     uint32_t* dense_code = nullptr;   // pattern -> order-preserving code (DenseSketchArgs, sketch.cuh)
     uint64_t* dense_hash = nullptr;   // the patterns' hashes in increasing order
@@ -514,25 +535,13 @@ struct ks_index {
     uint32_t* dense_flags = nullptr;  // device u32[4], table build: [0] table check, [3] largest rank of a pattern inside
                                       // its prefix group
     Buf b_dense_code, b_dense_hash, b_dense_group, b_dense_por, b_dense_flags, b_dense_work;
-    bool pending_dense = false;
-    bool scattered = false;  // the only batch was sketched straight into the regions of the unstable partition (pair_plan)
-    bool scatter_unchecked = false;  // ... and its count / zero-hash flag (d_count) have not been read yet: finalize does
-    PairSortPlan pair_plan;
+    PairSortPlan pair_plan;  // of a scattered batch
     Buf b_pair_work;
-    uint32_t build_path = 0;  // ks_stats.build_path of the last finalize
-    bool dense_sketched = false;  // pending batch: the rank kernel has already run over it (pipelined upload)
+    uint32_t build_path = 0;  // ks_stats.build_path of the last finalize (ks_index_clear keeps it)
     DenseSortPlan dense_plan;
     int dense_pid_bits = 0, dense_pos_bits = 0;
-    uint64_t* keys = nullptr;
-    uint32_t *key_grp = nullptr, *grp_start = nullptr, *t_size = nullptr, *t_abund = nullptr, *dir = nullptr;
-    uint64_t* d_counts = nullptr;
+    Csr csr;
     Buf b_keys, b_key_grp, b_grp_start, b_t_size, b_t_abund, b_dir, b_alt_hash, b_alt_loc, b_temp;
-    int dir_bits = 0, dir_shift = 0;
-    int dir_sub = DIR_SUB_COMPACT;  // layout of keys / key_grp / grp_start (index_build.cuh): compact, or segmented
-    uint32_t seg_nb = 0;
-    const uint32_t* seg_start = nullptr;  // (in the build's scratch, which stays with the handle until the next build)
-    const uint64_t* seg_counts = nullptr;
-    uint64_t U = 0, G = 0, n_ids = 0;
     // query path: per-handle scratch (grow-only) and a pinned word block for the counts the host reads back
     Buf b_q_ecount, b_q_pcount, b_q_hcount, b_q_sig, b_q_poff, b_q_hoff, b_q_ent_hash, b_q_ent_abund, b_q_win_key,
         b_q_win_hoff, b_q_stage, b_q_totals;
@@ -544,6 +553,7 @@ struct ks_index {
 
     void use() { KS_CUDA(cudaSetDevice(params.device)); }
     int end_bit() const { return 64 - lz; }
+    bool finalized() const { return state == Build::Finalized; }
 };
 
 namespace {
@@ -552,6 +562,7 @@ enum { EV_UP0, EV_UP1, EV_SK0, EV_SK1, EV_SO0, EV_SO1, EV_CS0, EV_CS1, EV_Q0, EV
 // pinned words of a handle: [0, QT_WORDS) totals of the query kernels; then this rank's header of a sharded search;
 // then every rank's header
 enum { HW_TOTALS = 0, HW_HDR = QT_WORDS, HW_ALL = QT_WORDS + 8, H_WORDS = QT_WORDS + 8 + 4 * MAX_SHARDS };
+static_assert(sizeof(StatusBlock) == 48 && sizeof(StatusBlock) <= QT_WORDS * 8, "the status block is read into the totals words");
 
 void ensure_ws(ks_index* x, size_t bytes) {
     if (bytes <= x->ws_bytes) return;
@@ -560,45 +571,52 @@ void ensure_ws(ks_index* x, size_t bytes) {
     x->ws_bytes = bytes;
 }
 
-void upload_batch(ks_index* x, DeviceBatch& b, const ks_proteome* p, bool allow_packed = false) {
-    const bool packed = allow_packed && p->packed && x->params.ksize <= (uint32_t)SK_MAX_TEMPLATE_K;
-    const uint64_t res_bytes = packed ? packed_bytes(p->n_res) : p->n_res + 64;
+// Buffers and shape of batch b for proteome p, its residues as 5-bit codes when `packed`; the caller copies the data in.
+void reserve_batch(ks_index* x, DeviceBatch& b, const ks_proteome* p, bool packed) {
     if (p->n_prot >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins in one batch");
-    if (res_bytes > b.res_cap) {
-        if (b.res) x->arena->release(b.res);
-        b.res_cap = res_bytes;
-        b.res = x->arena->alloc<uint8_t>(b.res_cap);
-    }
-    if (p->n_prot + 1 > b.offs_cap) {
-        if (b.offs) x->arena->release(b.offs);
-        b.offs_cap = p->n_prot + 1;
-        b.offs = x->arena->alloc<uint64_t>(b.offs_cap);
-    }
     b.packed = packed;
-    KS_CUDA(cudaMemcpyAsync(b.res, packed ? p->packed : p->residues, res_bytes, cudaMemcpyHostToDevice, x->stream));
-    KS_CUDA(cudaMemcpyAsync(b.offs, p->offsets, (p->n_prot + 1) * 8, cudaMemcpyHostToDevice, x->stream));
     b.n_prot = p->n_prot;
     b.n_res = p->n_res;
+    b.res = b.b_res.ensure<uint8_t>(x->arena, b.res_bytes());
+    b.offs = b.b_offs.ensure<uint64_t>(x->arena, p->n_prot + 1);
     proteome_shape(p, x->params.ksize, &b.n_windows, &b.max_len);
     b.valid = true;
 }
 
-void drop_csr(ks_index* x) {  // the buffers stay with the handle (grow-only), only the index state is dropped
-    x->keys = nullptr; x->key_grp = x->grp_start = x->t_size = x->t_abund = x->dir = nullptr; x->d_counts = nullptr;
-    x->finalized = false;
-    x->hash_col_valid = true;
-    x->dir_sub = DIR_SUB_COMPACT; x->seg_nb = 0; x->seg_start = nullptr; x->seg_counts = nullptr;
-    x->U = x->G = x->n_ids = 0;
+void upload_batch(ks_index* x, DeviceBatch& b, const ks_proteome* p, bool allow_packed = false) {
+    reserve_batch(x, b, p, allow_packed && p->packed && x->params.ksize <= (uint32_t)SK_MAX_TEMPLATE_K);
+    KS_CUDA(cudaMemcpyAsync(b.res, b.packed ? p->packed : p->residues, b.res_bytes(), cudaMemcpyHostToDevice, x->stream));
+    KS_CUDA(cudaMemcpyAsync(b.offs, p->offsets, (p->n_prot + 1) * 8, cudaMemcpyHostToDevice, x->stream));
 }
 
-void grow_tuples(ks_index* x, uint64_t need) {
+// The handle holds nothing afterwards (ks_index_clear, and a pending batch about to be sketched again).  The buffers stay
+// with the handle (grow-only), and so does build_path.
+void drop_content(ks_index* x) {
+    x->state = Build::Tuples;
+    x->csr = Csr();
+    x->n_tuples = x->n_prot = x->n_res = x->n_windows = 0;
+}
+
+// The resident batch has been added with n tuples and the handle now holds `state`: the one place a batch is counted.
+void commit_batch(ks_index* x, uint64_t n, Build state) {
+    const DeviceBatch& b = x->batch;
+    x->state = state;
+    x->n_tuples += n;
+    x->n_prot += b.n_prot;
+    x->n_res += b.n_res;
+    x->n_windows += b.n_windows;
+}
+
+// Room for `need` tuples.  keep = false: the tuples held are dropped (the buffers may be replaced without a copy).
+void grow_tuples(ks_index* x, uint64_t need, bool keep = true) {
     if (need <= x->cap) return;
-    uint64_t ncap = std::max<uint64_t>(need, x->n_tuples ? x->cap + x->cap / 2 : need);
+    const uint64_t held = keep ? x->n_tuples : 0;
+    uint64_t ncap = std::max<uint64_t>(need, held ? x->cap + x->cap / 2 : need);
     uint64_t* nh = x->arena->alloc<uint64_t>(ncap);
     uint64_t* nl = x->arena->alloc<uint64_t>(ncap);
-    if (x->n_tuples) {
-        KS_CUDA(cudaMemcpyAsync(nh, x->d_hash, x->n_tuples * 8, cudaMemcpyDeviceToDevice, x->stream));
-        KS_CUDA(cudaMemcpyAsync(nl, x->d_loc, x->n_tuples * 8, cudaMemcpyDeviceToDevice, x->stream));
+    if (held) {
+        KS_CUDA(cudaMemcpyAsync(nh, x->d_hash, held * 8, cudaMemcpyDeviceToDevice, x->stream));
+        KS_CUDA(cudaMemcpyAsync(nl, x->d_loc, held * 8, cudaMemcpyDeviceToDevice, x->stream));
     }
     if (x->d_hash) x->arena->release(x->d_hash);
     if (x->d_loc) x->arena->release(x->d_loc);
@@ -612,26 +630,44 @@ uint64_t expected_kept(const ks_index* x, uint64_t windows) {
     return std::min(windows, est);
 }
 
+// One status block read-back: its first `bytes` (the other words keep the values of `st`), and the unstable partition's
+// overflow flag into st.overflow when `part_overflow` is given.
+StatusBlock read_status(ks_index* x, const StatusBlock& st, size_t bytes, const uint32_t* part_overflow = nullptr) {
+    StatusBlock* h = (StatusBlock*)(x->h_words + HW_TOTALS);
+    *h = st;
+    KS_CUDA(cudaMemcpyAsync(h, x->d_status, bytes, cudaMemcpyDeviceToHost, x->stream));
+    if (part_overflow) KS_CUDA(cudaMemcpyAsync(&h->overflow, part_overflow, 4, cudaMemcpyDeviceToHost, x->stream));
+    KS_CUDA(cudaStreamSynchronize(x->stream));
+    return *h;
+}
+
+// A sketch launch over batch b: everything but the output (out_hash / out_loc / capacity, or the scatter), the tile range
+// and force_general, which callers set.  d_count / ws: the counter pair and workspace of the launch, the handle's own by
+// default.
+SketchArgs sketch_args(const ks_index* x, const DeviceBatch& b, uint32_t pid_base, uint64_t* d_count = nullptr, void* ws = nullptr) {
+    SketchArgs a;
+    a.residues = b.res; a.packed = b.packed ? 1 : 0; a.offsets = b.offs; a.n_res = b.n_res; a.n_prot = b.n_prot;
+    a.k = x->params.ksize; a.moltype = x->params.moltype; a.max_hash = x->max_hash; a.pid_base = pid_base;
+    a.out_hash = nullptr; a.out_loc = nullptr; a.capacity = 0;
+    a.d_count = d_count ? d_count : x->d_count; a.workspace = d_count ? ws : x->ws;
+    a.force_general = 0;
+    return a;
+}
+
 // Sketch batch `b` into (out_hash, out_loc) of `capacity`; returns the number of tuples the batch produces
 // (which may exceed capacity, in which case nothing past capacity was written).  d_count / ws: the counter pair and
 // workspace of the launch -- the handle's own for its batches, private ones for ks_sketch_batch and the query sketch (a
 // pipelined dense batch that is still pending keeps its counts in the handle's).
 uint64_t run_sketch(ks_index* x, const DeviceBatch& b, uint32_t pid_base, uint64_t* out_hash, uint64_t* out_loc,
                     uint64_t capacity, uint64_t* d_count = nullptr, void* ws = nullptr) {
-    if (!d_count) {
-        ensure_ws(x, sketch_workspace_bytes(b.n_res));
-        d_count = x->d_count;
-        ws = x->ws;
-    }
-    SketchArgs a;
-    a.residues = b.res; a.packed = b.packed ? 1 : 0; a.offsets = b.offs; a.n_res = b.n_res; a.n_prot = b.n_prot;
-    a.k = x->params.ksize; a.moltype = x->params.moltype; a.max_hash = x->max_hash; a.pid_base = pid_base;
-    a.out_hash = out_hash; a.out_loc = out_loc; a.capacity = capacity; a.d_count = d_count; a.workspace = ws;
+    if (!d_count) ensure_ws(x, sketch_workspace_bytes(b.n_res));
+    SketchArgs a = sketch_args(x, b, pid_base, d_count, ws);
+    a.out_hash = out_hash; a.out_loc = out_loc; a.capacity = capacity;
     a.force_general = x->hooks.sketch_general ? 1 : 0;  // test hook: exercise the look-back path at scaled == 1
     uint64_t r[2] = {0, 0};
     for (int attempt = 0; attempt < 2; attempt++) {
         KS_CUDA(launch_sketch(a, x->stream, &x->l_sketch));
-        KS_CUDA(cudaMemcpyAsync(r, d_count, 16, cudaMemcpyDeviceToHost, x->stream));
+        KS_CUDA(cudaMemcpyAsync(r, a.d_count, 16, cudaMemcpyDeviceToHost, x->stream));
         KS_CUDA(cudaStreamSynchronize(x->stream));
         if ((r[1] >> 32) == 0) break;  // no zero hash on the exact path
         a.force_general = 1;           // a hash of exactly 0 must be dropped: redo on the look-back path
@@ -648,19 +684,11 @@ int bits_for_value(uint64_t v) {  // bits needed to hold values 0 .. v
 // Dense k-mer space path (sketch_dense_kernel): the batch must be the index's only content, its k-mer space small and
 // well covered (otherwise the tables cost more than they save), and rank | protein | position must fit 64 bits.
 // KS_DENSE=0 switches the path off, KS_DENSE=1 drops the coverage condition (test hooks).
-bool dense_eligible_(const ks_index* x, const DeviceBatch& b, uint64_t n_prot_before, uint64_t n_tuples_before);
-bool dense_eligible(const ks_index* x, const DeviceBatch& b, uint64_t n_prot_before, uint64_t n_tuples_before) {
-    const bool e = dense_eligible_(x, b, n_prot_before, n_tuples_before);
-    if (x->hooks.timing) fprintf(stderr, "[ks] dense eligible: %d (state %d, prot before %llu, tuples before %llu, windows %llu)\n", (int)e,
-                                 x->dense_state, (unsigned long long)n_prot_before, (unsigned long long)n_tuples_before,
-                                 (unsigned long long)b.n_windows);
-    return e;
-}
-bool dense_eligible_(const ks_index* x, const DeviceBatch& b, uint64_t n_prot_before, uint64_t n_tuples_before) {
+bool dense_eligible(const ks_index* x, const DeviceBatch& b) {
     if (x->hooks.dense == 0) return false;
     const uint32_t k = x->params.ksize;
     if (x->params.moltype != KS_HP || k < (uint32_t)DENSE_MIN_K || k > (uint32_t)DENSE_MAX_K || x->max_hash != ~0ull) return false;
-    if (x->dense_state < 0 || n_prot_before || n_tuples_before || b.n_prot == 0 || b.n_res >= (1ull << 32)) return false;
+    if (x->dense_state < 0 || x->n_prot || x->n_tuples || b.n_prot == 0 || b.n_res >= (1ull << 32)) return false;
     if (x->hooks.dense != 1 && b.n_windows < (1ull << k) / 4) return false;
     // a key is code | protein | position; the code takes DENSE_PREFIX_BITS + rb bits (rb is known once the tables exist:
     // at most k + 1 when every pattern shared one hash prefix)
@@ -674,22 +702,6 @@ bool dense_eligible_(const ks_index* x, const DeviceBatch& b, uint64_t n_prot_be
     return code_bits + bits_for_value(b.n_prot - 1) + bits_for_value(b.max_len) <= 64;
 }
 
-void sketch_resident_general(ks_index* x);
-bool dense_begin(ks_index* x);
-void dense_rank_tiles(ks_index* x, uint32_t t0, uint32_t t1);
-
-// A batch deferred to finalize (dense path) is sketched the general way after all: something else is about to touch
-// the tuples or the resident batch.
-void materialize_pending(ks_index* x) {
-    if (!x->pending_dense && !x->scattered) return;
-    x->pending_dense = false;
-    x->dense_sketched = false;
-    x->scattered = false;  // the scattered tuples are dropped: the batch is sketched again, in order
-    x->scatter_unchecked = false;
-    x->n_tuples = x->n_prot = x->n_res = x->n_windows = 0;
-    sketch_resident_general(x);
-}
-
 // tuples per possible hash: distinct k-mers under this alphabet (hp k=24 has 2^24 of them for ~2*10^8 tuples on C2)
 double avg_postings(const ks_index* x, uint64_t n) {
     const double alphabet = x->params.moltype == KS_HP ? 2.0 : x->params.moltype == KS_DAYHOFF ? 6.0 : 20.0;
@@ -700,16 +712,28 @@ bool repeat_heavy(const ks_index* x, uint64_t n) { return avg_postings(x, n) > 0
 
 // Unstable partition of the general path (dense_scatter.cuh, PairSortPlan): the batch is the index's only content, hashes
 // rarely repeat (the bucket sort orders equal hashes by loc, pair by pair) and the tuple count fits two scatter levels.  KS_SCATTER=0 switches it off (test hook).
-bool scatter_eligible(const ks_index* x, const DeviceBatch& b, uint64_t n_prot_before, uint64_t n_tuples_before, PairSortPlan* plan) {
+bool scatter_eligible(const ks_index* x, const DeviceBatch& b, PairSortPlan* plan) {
     if (x->hooks.scatter_off) return false;
     if (x->params.ksize > (uint32_t)SK_MAX_TEMPLATE_K || x->hooks.sketch_general) return false;
-    if (n_prot_before || n_tuples_before || b.n_prot == 0 || b.n_windows > MAX_TUPLES) return false;
+    if (x->n_prot || x->n_tuples || b.n_prot == 0 || b.n_windows > MAX_TUPLES) return false;
     const uint64_t n_est = expected_kept(x, b.n_windows);  // exact for scaled == 1
     // measured: with hashes that repeat the stable path wins -- the C4 slice (protein k7 scaled 10, every hash twice on
     // average) takes 4.5 ms in the bin kernel with loc tie-breaks against 2.8 ms in the two-pass stable bucket sort
     if (repeat_heavy(x, n_est)) return false;
     *plan = pair_sort_plan(n_est, x->end_bit(), x->max_hash);
     return plan->custom != 0;
+}
+
+// How a batch of this shape is added to the handle, by the resident and the pipelined add alike: the dense k-mer space
+// path, the unstable partition of the general path (*plan), or the ordered sketch.
+enum class Route { Dense, Scatter, Ordered };
+Route choose_route(const ks_index* x, const DeviceBatch& b, PairSortPlan* plan) {
+    const bool dense = dense_eligible(x, b);
+    if (x->hooks.timing) fprintf(stderr, "[ks] dense eligible: %d (state %d, prot before %llu, tuples before %llu, windows %llu)\n", (int)dense,
+                                 x->dense_state, (unsigned long long)x->n_prot, (unsigned long long)x->n_tuples,
+                                 (unsigned long long)b.n_windows);
+    if (dense) return Route::Dense;
+    return scatter_eligible(x, b, plan) ? Route::Scatter : Route::Ordered;
 }
 
 void scatter_args(ks_index* x, SketchArgs* a) {
@@ -723,70 +747,27 @@ void scatter_args(ks_index* x, SketchArgs* a) {
     a->scatter.bits = pl.l1;
     a->scatter.lz = x->lz;
     a->scatter.overflow = (uint32_t*)(w + pl.off_overflow);
-    a->t_abund = x->max_hash != ~0ull ? x->t_abund : nullptr;
+    a->t_abund = x->max_hash != ~0ull ? (uint32_t*)x->b_t_abund.p : nullptr;
 }
 
 void scatter_begin(ks_index* x, const PairSortPlan& plan, uint64_t n_prot) {
     x->pair_plan = plan;
     char* w = x->b_pair_work.ensure<char>(x->arena, plan.bytes);
     KS_CUDA(cudaMemsetAsync(w + plan.off_small, 0, plan.small_bytes, x->stream));
-    if (x->max_hash != ~0ull) {  // scaled > 1: the sketch kernel counts the kept windows per protein
-        x->t_abund = x->b_t_abund.ensure<uint32_t>(x->arena, n_prot);
-        KS_CUDA(cudaMemsetAsync(x->t_abund, 0, n_prot * 4, x->stream));
+    if (x->max_hash != ~0ull) {  // scaled > 1: the sketch kernel counts the kept windows per protein (finalize's t_abund)
+        uint32_t* t_abund = x->b_t_abund.ensure<uint32_t>(x->arena, n_prot);
+        KS_CUDA(cudaMemsetAsync(t_abund, 0, n_prot * 4, x->stream));
     }
 }
 
-void sketch_resident(ks_index* x) {
-    DeviceBatch& b = x->batch;
-    if (!b.valid) fail(KS_ERR_VALIDATION, "Validation error: no batch is resident (call ks_index_upload first)");
-    if (x->finalized) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
-    materialize_pending(x);  // the resident batch was already added once and is being added again
-    if (dense_eligible(x, b, x->n_prot, x->n_tuples)) {
-        x->pending_dense = true;  // finalize builds the index from the resident residues in one go
-        x->n_tuples = b.n_windows; x->n_prot = b.n_prot; x->n_res = b.n_res; x->n_windows = b.n_windows;
-        return;
-    }
-    PairSortPlan plan;
-    if (scatter_eligible(x, b, x->n_prot, x->n_tuples, &plan)) {
-        scatter_begin(x, plan, b.n_prot);
-        ensure_ws(x, sketch_workspace_bytes(b.n_res));
-        SketchArgs a;
-        a.residues = b.res; a.packed = b.packed ? 1 : 0; a.offsets = b.offs; a.n_res = b.n_res; a.n_prot = b.n_prot;
-        a.k = x->params.ksize; a.moltype = x->params.moltype; a.max_hash = x->max_hash; a.pid_base = 0;
-        a.out_hash = nullptr; a.out_loc = nullptr; a.capacity = 0; a.d_count = x->d_count; a.workspace = x->ws;
-        a.force_general = 0;
-        scatter_args(x, &a);
-        KS_CUDA(cudaEventRecord(x->ev[EV_SK0], x->stream));
-        KS_CUDA(launch_sketch(a, x->stream, &x->l_sketch));
-        KS_CUDA(cudaEventRecord(x->ev[EV_SK1], x->stream));
-        x->t_sketch = true;
-        const bool exact = x->max_hash == ~0ull;
-        if (exact) {
-            // scaled == 1: the tuple count is known from the offsets; the kernel's own count and its zero-hash flag are
-            // read together with the build's results at the end of finalize (no host round trip here)
-            x->scattered = true;
-            x->scatter_unchecked = true;
-            x->n_tuples = b.n_windows; x->n_prot = b.n_prot; x->n_res = b.n_res; x->n_windows = b.n_windows;
-            return;
-        }
-        uint64_t r[2] = {0, 0};
-        KS_CUDA(cudaMemcpyAsync(r, x->d_count, 16, cudaMemcpyDeviceToHost, x->stream));
-        KS_CUDA(cudaStreamSynchronize(x->stream));
-        if (r[0] <= MAX_TUPLES) {
-            x->scattered = true;
-            x->n_tuples = r[0]; x->n_prot = b.n_prot; x->n_res = b.n_res; x->n_windows = b.n_windows;
-            return;
-        }
-        // a zero hash on the exact path (it must be dropped): the ordered path below
-    }
-    sketch_resident_general(x);
-}
+bool dense_begin(ks_index* x);
+void dense_rank_tiles(ks_index* x, uint32_t t0, uint32_t t1);
 
-void sketch_resident_general(ks_index* x) {
+// Ordered route: the resident batch (valid, the handle not finalized) sketched in (protein, pos) order behind the
+// tuples the handle holds.
+void sketch_ordered(ks_index* x) {
     DeviceBatch& b = x->batch;
-    if (!b.valid) fail(KS_ERR_VALIDATION, "Validation error: no batch is resident (call ks_index_upload first)");
     if (x->n_prot + b.n_prot >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins on one shard");
-    if (x->finalized) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
     grow_tuples(x, x->n_tuples + expected_kept(x, b.n_windows));
     KS_CUDA(cudaEventRecord(x->ev[EV_SK0], x->stream));
     uint64_t n = run_sketch(x, b, (uint32_t)x->n_prot, x->d_hash + x->n_tuples, x->d_loc + x->n_tuples, x->cap - x->n_tuples);
@@ -797,10 +778,52 @@ void sketch_resident_general(ks_index* x) {
     }
     KS_CUDA(cudaEventRecord(x->ev[EV_SK1], x->stream));
     x->t_sketch = true;
-    x->n_tuples += n;
-    x->n_prot += b.n_prot;
-    x->n_res += b.n_res;
-    x->n_windows += b.n_windows;
+    commit_batch(x, n, Build::Tuples);
+}
+
+// A pending batch is sketched again, in order: something else is about to touch the tuples or the resident batch, or
+// finalize found that its route does not apply after all.
+void materialize_pending(ks_index* x) {
+    if (x->state == Build::Tuples || x->finalized()) return;
+    drop_content(x);
+    sketch_ordered(x);
+}
+
+// Scatter route, after the sketch kernel: r = its count and zero-hash flag, or nullptr when they are read by finalize
+// (scaled == 1).  A zero hash on the exact path (it must be dropped), or more tuples than the partition takes, sends the
+// batch to the ordered route.
+void scatter_done(ks_index* x, const uint64_t* r) {
+    const DeviceBatch& b = x->batch;
+    if (!r) return commit_batch(x, b.n_windows, Build::ScatteredUnchecked);
+    const bool exact = x->max_hash == ~0ull;
+    if (exact ? ((r[1] >> 32) != 0 || r[0] != b.n_windows) : r[0] > MAX_TUPLES) return sketch_ordered(x);
+    commit_batch(x, r[0], Build::Scattered);
+}
+
+void sketch_resident(ks_index* x) {
+    DeviceBatch& b = x->batch;
+    if (!b.valid) fail(KS_ERR_VALIDATION, "Validation error: no batch is resident (call ks_index_upload first)");
+    if (x->finalized()) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
+    materialize_pending(x);  // the resident batch was already added once and is being added again
+    PairSortPlan plan;
+    const Route route = choose_route(x, b, &plan);
+    if (route == Route::Dense) return commit_batch(x, b.n_windows, Build::DenseDeferred);  // finalize builds it in one go
+    if (route == Route::Ordered) return sketch_ordered(x);
+    scatter_begin(x, plan, b.n_prot);
+    ensure_ws(x, sketch_workspace_bytes(b.n_res));
+    SketchArgs a = sketch_args(x, b, 0);
+    scatter_args(x, &a);
+    KS_CUDA(cudaEventRecord(x->ev[EV_SK0], x->stream));
+    KS_CUDA(launch_sketch(a, x->stream, &x->l_sketch));
+    KS_CUDA(cudaEventRecord(x->ev[EV_SK1], x->stream));
+    x->t_sketch = true;
+    // scaled == 1: the tuple count is known from the offsets; the kernel's own count and its zero-hash flag are read
+    // together with the build's results at the end of finalize (no host round trip here)
+    if (x->max_hash == ~0ull) return scatter_done(x, nullptr);
+    uint64_t r[2] = {0, 0};
+    KS_CUDA(cudaMemcpyAsync(r, x->d_count, 16, cudaMemcpyDeviceToHost, x->stream));
+    KS_CUDA(cudaStreamSynchronize(x->stream));
+    scatter_done(x, r);
 }
 
 // upload + sketch with the residues streamed in: the offsets go first (everything the tile -> protein map and
@@ -813,59 +836,37 @@ bool add_proteome_pipelined(ks_index* x, const ks_proteome* p) {
     if (x->params.ksize > (uint32_t)SK_MAX_TEMPLATE_K || x->hooks.no_pipeline)  // (test hook)
         return false;
     if (p->n_res < (64u << 20) || p->n_prot == 0) return false;  // small batches: one copy, one launch
-    if (x->finalized) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
+    if (x->finalized()) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
     materialize_pending(x);
-    bool dense = false, scat = false;  // dense k-mer space path / unstable partition of the general path
-    PairSortPlan scat_plan;
-    {   // a batch for the dense path: the rank kernel follows the chunks instead of the sketch kernel
-        DeviceBatch probe;
-        probe.n_prot = p->n_prot; probe.n_res = p->n_res;
-        proteome_shape(p, x->params.ksize, &probe.n_windows, &probe.max_len);
-        dense = dense_eligible(x, probe, x->n_prot, x->n_tuples);
-        if (!dense) scat = scatter_eligible(x, probe, x->n_prot, x->n_tuples, &scat_plan);
-    }
-    if (p->n_prot >= 0xffffffffull || x->n_prot + p->n_prot >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins on one shard");
+    if (x->n_prot + p->n_prot >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins on one shard");
     DeviceBatch& b = x->batch;
-    const bool packed = p->packed != nullptr;  // 5 bits per residue over PCIe instead of 8
-    const uint64_t res_bytes = packed ? packed_bytes(p->n_res) : p->n_res + 64;
-    const uint8_t* host_res = packed ? p->packed : p->residues;
-    const uint64_t tile_bytes = packed ? SK_TILE / 8 * 5 : SK_TILE;
-    if (res_bytes > b.res_cap) {
-        if (b.res) x->arena->release(b.res);
-        b.res_cap = res_bytes;
-        b.res = x->arena->alloc<uint8_t>(b.res_cap);
-    }
-    if (p->n_prot + 1 > b.offs_cap) {
-        if (b.offs) x->arena->release(b.offs);
-        b.offs_cap = p->n_prot + 1;
-        b.offs = x->arena->alloc<uint64_t>(b.offs_cap);
-    }
-    b.packed = packed;
-    b.n_prot = p->n_prot; b.n_res = p->n_res;
-    proteome_shape(p, x->params.ksize, &b.n_windows, &b.max_len);
-    b.valid = true;
-    if (!dense && !scat) grow_tuples(x, x->n_tuples + expected_kept(x, b.n_windows));
-    if (scat) scatter_begin(x, scat_plan, p->n_prot);
+    reserve_batch(x, b, p, p->packed != nullptr);  // 5 bits per residue over PCIe instead of 8
+    PairSortPlan plan;
+    Route route = choose_route(x, b, &plan);  // dense: the rank kernel follows the chunks instead of the sketch kernel
+    const uint8_t* host_res = b.packed ? p->packed : p->residues;
+    const uint64_t res_bytes = b.res_bytes();
+    const uint64_t tile_bytes = b.packed ? SK_TILE / 8 * 5 : SK_TILE;
+    if (route == Route::Ordered) grow_tuples(x, x->n_tuples + expected_kept(x, b.n_windows));
+    if (route == Route::Scatter) scatter_begin(x, plan, p->n_prot);
     ensure_ws(x, sketch_workspace_bytes(b.n_res));
     KS_CUDA(cudaEventRecord(x->ev[EV_UP0], x->stream));
     KS_CUDA(cudaEventRecord(x->ev[EV_SK0], x->stream));
     KS_CUDA(cudaMemcpyAsync(b.offs, p->offsets, (p->n_prot + 1) * 8, cudaMemcpyHostToDevice, x->stream));
-    if (dense && !dense_begin(x)) {  // the tables turned out unusable for this k: the general pipeline after all
-        dense = false;
-        x->n_tuples = 0;
-        grow_tuples(x, expected_kept(x, b.n_windows));
+    if (route == Route::Dense && !dense_begin(x)) {  // the tables turned out unusable for this k: the ordered route after all
+        route = Route::Ordered;
+        grow_tuples(x, x->n_tuples + expected_kept(x, b.n_windows));
     }
     // buffers were (re)allocated in compute-stream order: the copy stream must not run ahead of that
     KS_CUDA(cudaEventRecord(x->ev_chunk[CHUNKS], x->stream));
     KS_CUDA(cudaStreamWaitEvent(x->copy_stream, x->ev_chunk[CHUNKS], 0));
-    SketchArgs a;
-    a.residues = b.res; a.packed = packed ? 1 : 0; a.offsets = b.offs; a.n_res = b.n_res; a.n_prot = b.n_prot;
-    a.k = x->params.ksize; a.moltype = x->params.moltype; a.max_hash = x->max_hash; a.pid_base = (uint32_t)x->n_prot;
-    a.out_hash = x->d_hash + x->n_tuples; a.out_loc = x->d_loc + x->n_tuples; a.capacity = x->cap - x->n_tuples;
-    a.d_count = x->d_count; a.workspace = x->ws;
+    SketchArgs a = sketch_args(x, b, (uint32_t)x->n_prot);
     a.force_general = x->hooks.sketch_general ? 1 : 0;  // test hook: the look-back path at scaled == 1
-    if (scat) { a.out_hash = nullptr; a.out_loc = nullptr; a.capacity = 0; scatter_args(x, &a); }
-    if (!dense) KS_CUDA(launch_sketch_prepare(a, x->stream, &x->l_sketch));  // (dense_begin has done it)
+    if (route == Route::Scatter) {
+        scatter_args(x, &a);
+    } else {
+        a.out_hash = x->d_hash + x->n_tuples; a.out_loc = x->d_loc + x->n_tuples; a.capacity = x->cap - x->n_tuples;
+    }
+    if (route != Route::Dense) KS_CUDA(launch_sketch_prepare(a, x->stream, &x->l_sketch));  // (dense_begin has done it)
     const uint64_t nt = (b.n_res + SK_TILE - 1) / SK_TILE;
     const uint64_t per = (nt + CHUNKS - 1) / CHUNKS;
     for (int c = 0; c < CHUNKS; c++) {
@@ -877,65 +878,32 @@ bool add_proteome_pipelined(ks_index* x, const ks_proteome* p) {
         KS_CUDA(cudaEventRecord(x->ev_chunk[c], x->copy_stream));
         KS_CUDA(cudaStreamWaitEvent(x->stream, x->ev_chunk[c], 0));
         a.tile_begin = (uint32_t)t0; a.tile_end = (uint32_t)t1;
-        if (dense) dense_rank_tiles(x, (uint32_t)t0, (uint32_t)t1);
+        if (route == Route::Dense) dense_rank_tiles(x, (uint32_t)t0, (uint32_t)t1);
         else KS_CUDA(launch_sketch_tiles(a, x->stream, &x->l_sketch));
     }
-    if (dense) {  // finalize takes it from here (flags, second scatter level, buckets)
-        KS_CUDA(cudaEventRecord(x->ev[EV_UP1], x->stream));
-        KS_CUDA(cudaEventRecord(x->ev[EV_SK1], x->stream));
-        KS_CUDA(cudaStreamSynchronize(x->stream));
-        x->t_upload = x->t_sketch = true;
-        x->pending_dense = true;
-        x->dense_sketched = true;
-        x->n_tuples = b.n_windows; x->n_prot = b.n_prot; x->n_res = b.n_res; x->n_windows = b.n_windows;
-        return true;
-    }
-    KS_CUDA(launch_sketch_finish(a, x->stream));
     uint64_t r[2] = {0, 0};
-    KS_CUDA(cudaMemcpyAsync(r, x->d_count, 16, cudaMemcpyDeviceToHost, x->stream));
+    if (route != Route::Dense) {
+        KS_CUDA(launch_sketch_finish(a, x->stream));
+        KS_CUDA(cudaMemcpyAsync(r, x->d_count, 16, cudaMemcpyDeviceToHost, x->stream));
+    }
     KS_CUDA(cudaEventRecord(x->ev[EV_UP1], x->stream));
     KS_CUDA(cudaEventRecord(x->ev[EV_SK1], x->stream));
     KS_CUDA(cudaStreamSynchronize(x->stream));
     x->t_upload = x->t_sketch = true;
+    if (route == Route::Dense) commit_batch(x, b.n_windows, Build::DenseRanked);  // finalize takes it from here
+    else if (route == Route::Scatter) scatter_done(x, r);
     // a zero hash on the exact path, or more tuples than the estimate for scaled > 1 allowed for: redo the batch (now
-    // resident) through the plain path, which takes the look-back kernel / grows the buffer as needed
-    if (scat) {
-        const bool exact = x->max_hash == ~0ull;
-        if (exact ? ((r[1] >> 32) != 0 || r[0] != b.n_windows) : r[0] > MAX_TUPLES) {  // a zero hash: the ordered path
-            sketch_resident_general(x);
-            return true;
-        }
-        x->scattered = true;
-        x->n_tuples = r[0]; x->n_prot = b.n_prot; x->n_res = b.n_res; x->n_windows = b.n_windows;
-        return true;
-    }
-    if ((r[1] >> 32) != 0 || r[0] > x->cap - x->n_tuples) {
-        sketch_resident_general(x);
-        return true;
-    }
-    x->n_tuples += r[0];
-    x->n_prot += b.n_prot;
-    x->n_res += b.n_res;
-    x->n_windows += b.n_windows;
+    // resident) on the ordered route, which takes the look-back kernel / grows the buffer as needed
+    else if ((r[1] >> 32) != 0 || r[0] > x->cap - x->n_tuples) sketch_ordered(x);
+    else commit_batch(x, r[0], Build::Tuples);
     return true;
 }
 
-static double now_ms() {
-    struct timespec ts;
-    clock_gettime(CLOCK_MONOTONIC, &ts);
-    return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
-}
-
-CsrView view_of(const ks_index* x);
-
 // ---- dense path (sketch_dense_kernel, dense.cu) -------------------------------------------------------------------
 void dense_kernel_args(ks_index* x, SketchArgs* a, DenseSketchArgs* d) {
-    const DeviceBatch& b = x->batch;
     const DenseSortPlan& plan = x->dense_plan;
-    a->residues = b.res; a->packed = b.packed ? 1 : 0; a->offsets = b.offs; a->n_res = b.n_res; a->n_prot = b.n_prot;
-    a->k = x->params.ksize; a->moltype = x->params.moltype; a->max_hash = x->max_hash; a->pid_base = 0;
-    a->out_hash = nullptr; a->out_loc = nullptr; a->capacity = x->cap; a->d_count = x->d_count; a->workspace = x->ws;
-    a->force_general = 0;
+    *a = sketch_args(x, x->batch, 0);
+    a->capacity = x->cap;
     d->code_of_pattern = x->dense_code; d->out_keys = x->d_hash; d->pid_bits = x->dense_pid_bits; d->pos_bits = x->dense_pos_bits;
     d->sorted_hash = x->dense_hash; d->group_base = x->dense_group; d->rb = x->dense_rb; d->parity = x->dense_parity;
     d->exception_flag = (uint32_t*)(x->d_status + 4);
@@ -984,9 +952,7 @@ bool dense_begin(ks_index* x) {
     if (n > MAX_TUPLES) fail(KS_ERR_CAPACITY, "more than 2^31-1 tuples on one shard: shard the proteome over more GPUs");
     x->dense_pid_bits = bits_for_value(b.n_prot - 1);
     x->dense_pos_bits = bits_for_value(b.max_len);
-    x->n_tuples = 0;    // nothing is stored yet: the buffers may be replaced without a copy
-    grow_tuples(x, n);  // d_hash: the keys when the library sorts them; d_loc: the postings
-    x->n_tuples = n;
+    grow_tuples(x, n, false);  // d_hash: the keys when the library sorts them; d_loc: the postings
     // the key sort: hand-written (two scatter levels + a shared-memory sort per bucket) when the input fits its scheme,
     // the library's otherwise (KS_DENSE_SORT=library is a test hook)
     // layout of the keys: with the parity bit (exception windows handled) when code | protein | position fits 64 bits
@@ -1025,6 +991,26 @@ void dense_rank_tiles(ks_index* x, uint32_t t0, uint32_t t1) {
     KS_CUDA(launch_sketch_dense(a, d, x->stream, &x->l_sketch));
 }
 
+// The CSR's buffers for n tuples of P proteins.  The directory has about 4 tuples (<= 4 keys) per bucket, so that it stays
+// small next to the keys, and at least the 2^top_bits buckets of the key sort (a directory bucket must not span two of
+// them); the key, group and directory arrays get `slack` more slots.
+Csr reserve_csr(ks_index* x, uint64_t n, uint32_t P, int top_bits, uint64_t slack) {
+    int bits = 8;
+    while (bits < 24 && (4ull << bits) < n) bits++;
+    Arena* ar = x->arena;
+    Csr c;
+    c.dir_bits = std::max(bits, top_bits);
+    c.dir_shift = 64 - x->lz - c.dir_bits;
+    c.t_abund = x->b_t_abund.ensure<uint32_t>(ar, P);
+    c.t_size = x->b_t_size.ensure<uint32_t>(ar, P);
+    c.keys = x->b_keys.ensure<uint64_t>(ar, n + slack);
+    c.key_grp = x->b_key_grp.ensure<uint32_t>(ar, n + slack);
+    c.grp_start = x->b_grp_start.ensure<uint32_t>(ar, n + slack);
+    c.dir = x->b_dir.ensure<uint32_t>(ar, (1ull << c.dir_bits) + slack);
+    c.d_counts = x->d_status;
+    return c;
+}
+
 // Build the index of the pending batch on the dense path.  Returns false (nothing changed that matters) when the path
 // turns out not to apply: the tables are unusable for this k, a window holds a residue of neither hp class, or heavy
 // repeats of one k-mer overflowed a sort bucket.
@@ -1032,39 +1018,23 @@ bool dense_finalize(ks_index* x) {
     DeviceBatch& b = x->batch;
     const uint32_t k = x->params.ksize;
     Arena* ar = x->arena;
-    if (!x->dense_sketched) {
+    if (x->state == Build::DenseDeferred) {
         KS_CUDA(cudaEventRecord(x->ev[EV_SK0], x->stream));
         if (!dense_begin(x)) return false;
         dense_rank_tiles(x, 0, 0);
         KS_CUDA(cudaEventRecord(x->ev[EV_SK1], x->stream));
     }
-    x->dense_sketched = false;
     const uint64_t n = b.n_windows;
     const uint32_t P = (uint32_t)b.n_prot;
     const DenseSortPlan plan = x->dense_plan;
     char* work = (char*)x->b_dense_work.p;
     // No host round trip between the rank kernel and the CSR: the kernels read the rank kernel's flags on the device, and
     // everything the host has to know (flags, counts, overflow) comes back in ONE read at the end.
-    int bits = 8;  // directory as on the general path
-    while (bits < 24 && (4ull << bits) < n) bits++;
-    if (plan.custom && plan.total > bits) bits = plan.total;  // a directory bucket never spans two sort buckets
     const uint64_t slack = (plan.custom ? (1ull << plan.total) : 0) + 2;  // segmented layout: a sentinel slot per bucket
-    x->dir_bits = bits;
-    x->dir_shift = 64 - x->lz - bits;
-    x->t_abund = x->b_t_abund.ensure<uint32_t>(ar, P);
-    x->t_size = x->b_t_size.ensure<uint32_t>(ar, P);
-    x->keys = x->b_keys.ensure<uint64_t>(ar, n + slack);
-    x->key_grp = x->b_key_grp.ensure<uint32_t>(ar, n + slack);
-    x->grp_start = x->b_grp_start.ensure<uint32_t>(ar, n + slack);
-    x->dir = x->b_dir.ensure<uint32_t>(ar, (1ull << bits) + slack);
-    x->d_counts = x->d_status;
-    int out_dir_sub = DIR_SUB_COMPACT;
-    uint32_t out_seg_nb = 0;
-    const uint32_t* out_seg_start = nullptr;
-    const uint64_t* out_seg_counts = nullptr;
+    Csr cs = reserve_csr(x, n, P, plan.custom ? plan.total : 0, slack);
     DenseCsrArgs c;
-    c.dir = x->dir; c.dir_bits = bits;
-    c.out_dir_sub = &out_dir_sub; c.out_seg_nb = &out_seg_nb; c.out_seg_start = &out_seg_start; c.out_seg_counts = &out_seg_counts;
+    c.dir = cs.dir; c.dir_bits = cs.dir_bits;
+    c.out_dir_sub = &cs.dir_sub; c.out_seg_nb = &cs.seg_nb; c.out_seg_start = &cs.seg_start; c.out_seg_counts = &cs.seg_counts;
     c.plan = plan; c.work = work;
     c.keys_a = x->d_hash; c.keys_b = plan.custom ? nullptr : x->b_alt_hash.ensure<uint64_t>(ar, n);
     c.n = n; c.n_prot = P; c.k = k;
@@ -1074,133 +1044,98 @@ bool dense_finalize(ks_index* x) {
     c.residues = b.res; c.packed = b.packed ? 1 : 0;
     c.skip_flag = (uint32_t*)(x->d_status + 4); c.exc_flag = c.skip_flag + 1; c.overflow = (uint32_t*)(x->d_status + 5);
     c.counts_zeroed = 1;
-    c.loc = x->d_loc; c.keys = x->keys; c.key_grp = x->key_grp; c.grp_start = x->grp_start;
-    c.t_size = x->t_size; c.t_abund = x->t_abund; c.d_counts = x->d_counts;
+    c.loc = x->d_loc; c.keys = cs.keys; c.key_grp = cs.key_grp; c.grp_start = cs.grp_start;
+    c.t_size = cs.t_size; c.t_abund = cs.t_abund; c.d_counts = cs.d_counts;
     c.temp_bytes = dense_csr_temp_bytes(n);
     c.temp = x->b_temp.ensure<char>(ar, c.temp_bytes);
     c.ev_sorted = x->ev[EV_PART];
     KS_CUDA(cudaEventRecord(x->ev[EV_SO0], x->stream));
     KS_CUDA(dense_build_csr(c, x->stream, &x->l_sort, &x->l_csr));
     KS_CUDA(cudaEventRecord(x->ev[EV_SO1], x->stream));
-    if (out_dir_sub == DIR_SUB_COMPACT) {  // library-sorted keys: compact layout, the directory in its own pass
-        KS_CUDA(launch_directory(x->keys, x->d_counts, x->dir, x->dir_bits, x->dir_shift, x->stream));
+    if (cs.dir_sub == DIR_SUB_COMPACT) {  // library-sorted keys: compact layout, the directory in its own pass
+        KS_CUDA(launch_directory(cs.keys, cs.d_counts, cs.dir, cs.dir_bits, cs.dir_shift, x->stream));
         x->l_csr += 1;
     }
     KS_CUDA(cudaEventRecord(x->ev[EV_CS1], x->stream));
-    // (the bucket tables of the segmented layout live in the work buffer, which stays with the handle until the next build)
-    x->seg_start = out_seg_start; x->seg_counts = out_seg_counts;
     x->t_sketch = x->t_sort = x->t_csr = true;
-    uint64_t st[6];  // the status block: [0..1] counts, [2] produced, [3] zero-hash flag, [4] flags, [5] overflow
-    uint64_t* hwp = x->h_words + HW_TOTALS;
-    KS_CUDA(cudaMemcpyAsync(hwp, x->d_status, 48, cudaMemcpyDeviceToHost, x->stream));
-    KS_CUDA(cudaStreamSynchronize(x->stream));
-    memcpy(st, hwp, sizeof(st));
-    uint64_t hw[5] = {st[0], st[1], st[2], st[4], st[5]};
-    const uint32_t unhandled = (uint32_t)hw[3];  // [0] of the pair: an exception the path does not handle, or a zero hash
+    const StatusBlock st = read_status(x, StatusBlock{}, sizeof(StatusBlock));
+    const uint32_t unhandled = (uint32_t)st.dense_flags;  // an exception the path does not handle, or a zero hash
     if (x->hooks.timing)
         fprintf(stderr, "[ks] dense finalize: n %llu produced %llu unhandled %u exc %u overflow %u U %llu G %llu plan l1 %d l2 %d rb %d\n",
-                (unsigned long long)n, (unsigned long long)hw[2], unhandled, (uint32_t)(hw[3] >> 32), (uint32_t)hw[4],
-                (unsigned long long)hw[0], (unsigned long long)hw[1], plan.l1, plan.l2, x->dense_rb);
+                (unsigned long long)n, (unsigned long long)st.produced, unhandled, (uint32_t)(st.dense_flags >> 32),
+                (uint32_t)st.overflow, (unsigned long long)st.U, (unsigned long long)st.G, plan.l1, plan.l2, x->dense_rb);
     if (unhandled) return false;
-    if (hw[2] != n) fail(KS_ERR_CUDA, "internal error: dense path produced an unexpected number of tuples");
-    if ((uint32_t)hw[4]) return false;  // heavy repeats of one k-mer overflowed a sort bucket: the general path handles those
-    x->U = hw[0]; x->G = hw[1];
-    x->dir_sub = out_dir_sub; x->seg_nb = out_seg_nb;
-    x->hash_col_valid = false;  // d_hash holds code keys: the sorted hash column is rebuilt from the CSR on demand
+    if (st.produced != n) fail(KS_ERR_CUDA, "internal error: dense path produced an unexpected number of tuples");
+    if ((uint32_t)st.overflow) return false;  // heavy repeats of one k-mer overflowed a sort bucket: the general path handles those
+    cs.U = st.U; cs.G = st.G;
+    cs.hash_col_valid = false;  // d_hash holds code keys: the sorted hash column is rebuilt from the CSR on demand
+    x->csr = cs;
     x->build_path = plan.custom ? 1u : 2u;
-    x->pending_dense = false;
-    x->finalized = true;
+    x->state = Build::Finalized;
     return true;
 }
 
 void finalize(ks_index* x) {
-    if (x->finalized) return;
-    if (x->pending_dense) {
+    if (x->finalized()) return;
+    if (x->state == Build::DenseDeferred || x->state == Build::DenseRanked) {
         if (dense_finalize(x)) return;
         materialize_pending(x);  // not applicable after all: the general path from here on
     }
     const bool dbg = x->hooks.timing;
-    double t0 = dbg ? now_ms() : 0;
+    double t0 = dbg ? wall_ms() : 0;
     const uint64_t n = x->n_tuples;
     if (n > MAX_TUPLES) fail(KS_ERR_CAPACITY, "more than 2^31-1 tuples on one shard: shard the proteome over more GPUs");
     const uint32_t P = (uint32_t)x->n_prot;
-    int bits = 8;  // ~4 tuples (<= 4 keys) per directory bucket: the table stays small next to the keys
-    while (bits < 24 && (4ull << bits) < n) bits++;
+    const bool scattered = x->state == Build::Scattered || x->state == Build::ScatteredUnchecked;
     // the bucket sort writes the CSR in the segmented layout: a directory bucket must not span two sort buckets, and the
     // key / group arrays carry one sentinel slot per sort bucket
-    const int top_bits = x->scattered ? x->pair_plan.total : build_top_bits(n, x->end_bit(), x->max_hash, avg_postings(x, n));
-    if (top_bits > bits) bits = top_bits;
+    const int top_bits = scattered ? x->pair_plan.total : build_top_bits(n, x->end_bit(), x->max_hash, avg_postings(x, n));
     const uint64_t slack = std::max<uint64_t>(build_slack(n), top_bits > 0 ? (1ull << top_bits) + 2 : 2);
-    x->dir_bits = bits;
-    x->dir_shift = 64 - x->lz - bits;
+    Csr cs = reserve_csr(x, n, P, top_bits, slack);
     Arena* ar = x->arena;
-    x->t_abund = x->b_t_abund.ensure<uint32_t>(ar, P);
-    x->t_size = x->b_t_size.ensure<uint32_t>(ar, P);
-    x->keys = x->b_keys.ensure<uint64_t>(ar, n + slack);
-    x->key_grp = x->b_key_grp.ensure<uint32_t>(ar, n + slack);
-    x->grp_start = x->b_grp_start.ensure<uint32_t>(ar, n + slack);
-    x->dir = x->b_dir.ensure<uint32_t>(ar, (1ull << bits) + slack);
-    x->d_counts = x->d_status;
     // the second tuple pair is the sort's ping-pong partner; a scattered batch has its regions instead
-    uint64_t* hb = x->scattered ? nullptr : x->b_alt_hash.ensure<uint64_t>(ar, n);
-    uint64_t* lb = x->scattered ? nullptr : x->b_alt_loc.ensure<uint64_t>(ar, n);
+    uint64_t* hb = scattered ? nullptr : x->b_alt_hash.ensure<uint64_t>(ar, n);
+    uint64_t* lb = scattered ? nullptr : x->b_alt_loc.ensure<uint64_t>(ar, n);
+    if (scattered) grow_tuples(x, n, false);  // the tuples sit in the regions of the unstable partition; the postings go to d_loc
     BuildArgs a;
     a.hash_a = x->d_hash; a.loc_a = x->d_loc; a.hash_b = hb; a.loc_b = lb;
     a.n = n; a.n_prot = P; a.end_bit = x->end_bit(); a.max_hash = x->max_hash;
     a.repeat_heavy = repeat_heavy(x, n) ? 1 : 0;  // measured: the bin kernel only wins when repeats are rare
     a.ls_variant = x->hooks.ls_variant;
     a.avg_postings = avg_postings(x, n);
-    int out_dir_sub = DIR_SUB_COMPACT;
-    uint32_t out_seg_nb = 0;
-    const uint32_t* out_seg_start = nullptr;
-    const uint64_t* out_seg_counts = nullptr;
-    a.out_dir_sub = &out_dir_sub; a.out_seg_nb = &out_seg_nb; a.out_seg_start = &out_seg_start; a.out_seg_counts = &out_seg_counts;
+    a.out_dir_sub = &cs.dir_sub; a.out_seg_nb = &cs.seg_nb; a.out_seg_start = &cs.seg_start; a.out_seg_counts = &cs.seg_counts;
     const uint32_t* d_overflow = nullptr;  // device flag of the unstable partition (a region overflowed)
-    if (x->scattered) {  // the tuples sit in the regions of the unstable partition; the postings go to d_loc
-        x->n_tuples = 0;
-        grow_tuples(x, n);
-        x->n_tuples = n;
-        a.loc_a = x->d_loc; a.hash_a = x->d_hash;
+    if (scattered) {
         a.plan = x->pair_plan; a.work = x->b_pair_work.p; a.offsets = x->batch.offs; a.k = x->params.ksize;
         a.overflow_dev = &d_overflow;
         a.abund_ready = x->max_hash != ~0ull ? 1 : 0;
     }
-    a.keys = x->keys; a.key_grp = x->key_grp; a.grp_start = x->grp_start; a.t_size = x->t_size; a.t_abund = x->t_abund;
-    a.d_counts = x->d_counts; a.dir = x->dir; a.dir_bits = x->dir_bits; a.dir_shift = x->dir_shift;
+    a.keys = cs.keys; a.key_grp = cs.key_grp; a.grp_start = cs.grp_start; a.t_size = cs.t_size; a.t_abund = cs.t_abund;
+    a.d_counts = cs.d_counts; a.dir = cs.dir; a.dir_bits = cs.dir_bits; a.dir_shift = cs.dir_shift;
     a.temp_bytes = build_temp_bytes(n, x->end_bit());
     a.temp = x->b_temp.ensure<char>(ar, a.temp_bytes);
     a.ev_sorted = x->ev[EV_SO1];
     a.ev_partitioned = x->ev[EV_PART];
     int in_a = 1, hash_written = 1;
     a.hash_written = &hash_written;
-    double t1 = dbg ? now_ms() : 0;
+    double t1 = dbg ? wall_ms() : 0;
     KS_CUDA(cudaEventRecord(x->ev[EV_SO0], x->stream));
     KS_CUDA(build_index(a, x->stream, &in_a, &x->l_sort, &x->l_csr));
     KS_CUDA(cudaEventRecord(x->ev[EV_CS1], x->stream));
-    x->dir_sub = out_dir_sub;
-    x->seg_nb = out_seg_nb;
-    // (the bucket tables of the segmented layout live in scratch that stays with the handle until the next build)
-    x->seg_start = out_seg_start; x->seg_counts = out_seg_counts;
-    const bool was_scattered = x->scattered;
-    double t2 = dbg ? now_ms() : 0;
+    double t2 = dbg ? wall_ms() : 0;
     x->t_sort = x->t_csr = true;
     // everything the host has to know comes back in ONE read: the CSR totals, and for a scattered batch the partition's
     // overflow flag and (when the sketch was not checked yet) the sketch kernel's count and zero-hash flag
-    uint64_t* hw = x->h_words + HW_TOTALS;
-    hw[2] = n; hw[3] = 0; hw[4] = 0;
-    // (d_counts and d_count are neighbours in the status block)
-    KS_CUDA(cudaMemcpyAsync(hw, x->d_status, x->scatter_unchecked ? 32 : 16, cudaMemcpyDeviceToHost, x->stream));
-    if (d_overflow) KS_CUDA(cudaMemcpyAsync(hw + 4, d_overflow, 4, cudaMemcpyDeviceToHost, x->stream));
-    KS_CUDA(cudaStreamSynchronize(x->stream));
-    if (was_scattered && ((uint32_t)hw[4] != 0 || hw[2] != n || (hw[3] >> 32) != 0)) {
+    StatusBlock st{};
+    st.produced = n;
+    st = read_status(x, st, x->state == Build::ScatteredUnchecked ? 32 : 16, d_overflow);
+    if (scattered && ((uint32_t)st.overflow != 0 || st.produced != n || (st.zero_flag >> 32) != 0)) {
         // a k-mer repeated thousands of times filled a region, or a window hashed to exactly 0 (it must be dropped):
         // sketch again in order, stable partition
         materialize_pending(x);
         finalize(x);
         return;
     }
-    x->scattered = false;
-    x->scatter_unchecked = false;
     if (!in_a) {  // the sorted tuples sit in the alternate pair: swap roles, nothing is freed
         std::swap(x->d_hash, hb); std::swap(x->d_loc, lb);
         const size_t cap_bytes = x->cap * 8;
@@ -1208,19 +1143,21 @@ void finalize(ks_index* x) {
         x->b_alt_hash.p = hb; x->b_alt_hash.bytes = cap_bytes;
         x->b_alt_loc.p = lb; x->b_alt_loc.bytes = cap_bytes;
     }
-    x->U = hw[0]; x->G = hw[1];
-    x->hash_col_valid = hash_written != 0;
-    x->build_path = was_scattered ? 3u : 0u;
-    x->finalized = true;
-    if (dbg) fprintf(stderr, "[ks] finalize: alloc %.3f ms, build_index (host) %.3f ms, tail %.3f ms\n", t1 - t0, t2 - t1, now_ms() - t2);
+    cs.U = st.U; cs.G = st.G;
+    cs.hash_col_valid = hash_written != 0;
+    x->csr = cs;
+    x->build_path = scattered ? 3u : 0u;
+    x->state = Build::Finalized;
+    if (dbg) fprintf(stderr, "[ks] finalize: alloc %.3f ms, build_index (host) %.3f ms, tail %.3f ms\n", t1 - t0, t2 - t1, wall_ms() - t2);
 }
 
 CsrView view_of(const ks_index* x) {
+    const Csr& c = x->csr;
     CsrView v;
-    v.hash = x->d_hash; v.loc = x->d_loc; v.keys = x->keys; v.key_grp = x->key_grp; v.grp_start = x->grp_start;
-    v.t_size = x->t_size; v.t_abund = x->t_abund; v.dir = x->dir; v.d_counts = x->d_counts; v.n = x->n_tuples;
-    v.n_prot = (uint32_t)x->n_prot; v.dir_bits = x->dir_bits; v.dir_shift = x->dir_shift;
-    v.dir_sub = x->dir_sub; v.seg_nb = x->seg_nb; v.seg_start = x->seg_start; v.seg_counts = x->seg_counts;
+    v.hash = x->d_hash; v.loc = x->d_loc; v.keys = c.keys; v.key_grp = c.key_grp; v.grp_start = c.grp_start;
+    v.t_size = c.t_size; v.t_abund = c.t_abund; v.dir = c.dir; v.d_counts = c.d_counts; v.n = x->n_tuples;
+    v.n_prot = (uint32_t)x->n_prot; v.dir_bits = c.dir_bits; v.dir_shift = c.dir_shift;
+    v.dir_sub = c.dir_sub; v.seg_nb = c.seg_nb; v.seg_start = c.seg_start; v.seg_counts = c.seg_counts;
     return v;
 }
 
@@ -1364,12 +1301,7 @@ ks_status ks_index_finalize(ks_index* x) {
 ks_status ks_index_clear(ks_index* x) {
     return guarded([&] {
         x->use();
-        drop_csr(x);
-        x->pending_dense = false;
-        x->dense_sketched = false;
-        x->scattered = false;
-        x->scatter_unchecked = false;
-        x->n_tuples = 0; x->n_prot = 0; x->n_res = 0; x->n_windows = 0;
+        drop_content(x);
     });
 }
 ks_status ks_index_process_fasta(ks_index* x, const char* path, uint64_t ambig_seed) {
@@ -1394,7 +1326,7 @@ ks_status ks_index_add_tuples(ks_index* x, const uint64_t* hash, const uint32_t*
             loc[i] = ((uint64_t)(pid[i] + (uint32_t)x->n_prot) << 32) | pos[i];
             if (i && loc[i] <= loc[i - 1]) fail(KS_ERR_VALIDATION, "Validation error: tuples must be ordered by (protein, pos)");
         }
-        if (x->finalized) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
+        if (x->finalized()) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
         grow_tuples(x, x->n_tuples + n);
         if (n) {
             KS_CUDA(cudaMemcpyAsync(x->d_hash + x->n_tuples, hash, n * 8, cudaMemcpyHostToDevice, x->stream));
@@ -1413,7 +1345,7 @@ ks_status ks_index_stats(ks_index* x, ks_stats* out) {
         KS_CUDA(cudaStreamSynchronize(x->stream));
         ks_stats s{};
         s.n_proteins = x->n_prot; s.n_residues = x->n_res; s.n_windows = x->n_windows; s.n_tuples = x->n_tuples;
-        s.n_unique_hashes = x->U; s.n_groups = x->G; s.n_distinct_ids = x->n_ids; s.device_bytes = x->live_bytes;
+        s.n_unique_hashes = x->csr.U; s.n_groups = x->csr.G; s.n_distinct_ids = x->csr.n_ids; s.device_bytes = x->live_bytes;
         s.sketch_launches = x->l_sketch; s.sort_launches = x->l_sort; s.csr_launches = x->l_csr; s.search_launches = x->l_search;
         if (x->t_upload) KS_CUDA(cudaEventElapsedTime(&s.ms_upload, x->ev[EV_UP0], x->ev[EV_UP1]));
         if (x->t_sketch) KS_CUDA(cudaEventElapsedTime(&s.ms_sketch, x->ev[EV_SK0], x->ev[EV_SK1]));
@@ -1424,7 +1356,7 @@ ks_status ks_index_stats(ks_index* x, ks_stats* out) {
         }
         if (x->t_csr) KS_CUDA(cudaEventElapsedTime(&s.ms_csr, x->ev[EV_SO1], x->ev[EV_CS1]));
         s.ms_search = x->ms_search;
-        s.finalized = x->finalized ? 1 : 0;
+        s.finalized = x->finalized() ? 1 : 0;
         s.build_path = x->build_path;
         *out = s;
     });
@@ -1436,7 +1368,7 @@ ks_status ks_index_stats(ks_index* x, ks_stats* out) {
 ks_status ks_index_signature_count(ks_index* x, uint64_t* out) {
     return guarded([&] {
         if (!x || !out) fail(KS_ERR_VALIDATION, "Validation error: null argument");
-        if (!x->finalized) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
         x->use();
         const uint64_t P = x->n_prot;
         std::vector<uint64_t> sums(P ? P : 1, 0);
@@ -1444,13 +1376,13 @@ ks_status ks_index_signature_count(ks_index* x, uint64_t* out) {
             Arena tmp(x->stream, &x->live_bytes);
             unsigned long long* d = (unsigned long long*)tmp.alloc<uint64_t>(P);
             KS_CUDA(cudaMemsetAsync(d, 0, P * 8, x->stream));
-            KS_CUDA(launch_id_sums(view_of(x), x->U, d, x->stream));
+            KS_CUDA(launch_id_sums(view_of(x), x->csr.U, d, x->stream));
             KS_CUDA(cudaMemcpyAsync(sums.data(), d, P * 8, cudaMemcpyDeviceToHost, x->stream));
             KS_CUDA(cudaStreamSynchronize(x->stream));
         }
         std::sort(sums.begin(), sums.begin() + P);
-        x->n_ids = (uint64_t)(std::unique(sums.begin(), sums.begin() + P) - sums.begin());
-        *out = x->n_ids;
+        x->csr.n_ids = (uint64_t)(std::unique(sums.begin(), sums.begin() + P) - sums.begin());
+        *out = x->csr.n_ids;
     });
 }
 
@@ -1464,10 +1396,10 @@ ks_status ks_sketch_batch(ks_index* x, const ks_proteome* p, ks_sketch** out) {
         // a private batch: the index's resident batch and tuples are left alone
         b.res = keep.alloc<uint8_t>(p->n_res + 64);
         b.offs = keep.alloc<uint64_t>(p->n_prot + 1);
-        b.res_cap = p->n_res + 64; b.offs_cap = p->n_prot + 1;
         KS_CUDA(cudaMemcpyAsync(b.res, p->residues, p->n_res + 64, cudaMemcpyHostToDevice, x->stream));
         KS_CUDA(cudaMemcpyAsync(b.offs, p->offsets, (p->n_prot + 1) * 8, cudaMemcpyHostToDevice, x->stream));
-        b.n_prot = p->n_prot; b.n_res = p->n_res; b.n_windows = count_windows(p->offsets, p->n_prot, x->params.ksize);
+        b.n_prot = p->n_prot; b.n_res = p->n_res;
+        proteome_shape(p, x->params.ksize, &b.n_windows, &b.max_len);
         b.valid = true;
         const uint64_t cap = b.n_windows;
         uint64_t* h = keep.alloc<uint64_t>(cap);
@@ -1484,13 +1416,13 @@ ks_status ks_sketch_batch(ks_index* x, const ks_proteome* p, ks_sketch** out) {
 ks_status ks_index_export(ks_index* x, ks_sketch** out) {
     return guarded([&] {
         if (!x || !out) fail(KS_ERR_VALIDATION, "Validation error: null argument");
-        if (!x->finalized) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
         x->use();
         Arena keep(x->stream, &x->live_bytes), tmp(x->stream, &x->live_bytes);
         Grouped g;
-        if (!x->hash_col_valid) {
+        if (!x->csr.hash_col_valid) {
             KS_CUDA(expand_sorted_hash(view_of(x), x->d_hash, x->stream));
-            x->hash_col_valid = true;
+            x->csr.hash_col_valid = true;
         }
         group_by_owner(keep, tmp, x->d_hash, x->d_loc, x->n_tuples, (uint32_t)x->n_prot, x->end_bit(), &g, &x->l_csr);
         *out = sketch_to_host(g, x->d_hash, x->d_loc, x->n_tuples, x->n_prot, x->stream);
@@ -1506,37 +1438,37 @@ void ks_sketch_free(ks_sketch* s) {
 ks_status ks_index_csr(ks_index* x, ks_csr** out) {
     return guarded([&] {
         if (!x || !out) fail(KS_ERR_VALIDATION, "Validation error: null argument");
-        if (!x->finalized) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
         x->use();
         ks_csr* c = (ks_csr*)calloc(1, sizeof(ks_csr));
         if (!c) throw std::bad_alloc();
-        c->n_keys = x->U; c->n_postings = x->n_tuples;
-        const bool seg = x->dir_sub != DIR_SUB_COMPACT;
-        const uint64_t span = seg ? x->n_tuples + x->seg_nb + 1 : x->U + 1;  // key / group positions in use
-        uint64_t* keys = to_host(x->keys, seg ? span : x->U, x->stream);
-        uint32_t* kg = to_host(x->key_grp, span, x->stream);
-        uint32_t* gs = to_host(x->grp_start, seg ? span : x->G + 1, x->stream);
+        c->n_keys = x->csr.U; c->n_postings = x->n_tuples;
+        const bool seg = x->csr.dir_sub != DIR_SUB_COMPACT;
+        const uint64_t span = seg ? x->n_tuples + x->csr.seg_nb + 1 : x->csr.U + 1;  // key / group positions in use
+        uint64_t* keys = to_host(x->csr.keys, seg ? span : x->csr.U, x->stream);
+        uint32_t* kg = to_host(x->csr.key_grp, span, x->stream);
+        uint32_t* gs = to_host(x->csr.grp_start, seg ? span : x->csr.G + 1, x->stream);
         uint64_t* loc = to_host(x->d_loc, x->n_tuples, x->stream);
-        uint32_t* st = seg ? to_host(x->seg_start, (uint64_t)x->seg_nb + 1, x->stream) : nullptr;
-        uint64_t* sc = seg ? to_host(x->seg_counts, x->seg_nb, x->stream) : nullptr;
+        uint32_t* st = seg ? to_host(x->csr.seg_start, (uint64_t)x->csr.seg_nb + 1, x->stream) : nullptr;
+        uint64_t* sc = seg ? to_host(x->csr.seg_counts, x->csr.seg_nb, x->stream) : nullptr;
         KS_CUDA(cudaStreamSynchronize(x->stream));
-        c->row_ptr = (uint64_t*)malloc((x->U + 1) * 8);
+        c->row_ptr = (uint64_t*)malloc((x->csr.U + 1) * 8);
         c->pid = (uint32_t*)malloc((x->n_tuples ? x->n_tuples : 1) * 4);
         c->pos = (uint32_t*)malloc((x->n_tuples ? x->n_tuples : 1) * 4);
         if (!c->row_ptr || !c->pid || !c->pos) throw std::bad_alloc();
         if (!seg) {
             c->keys = keys;
-            for (uint64_t u = 0; u <= x->U; u++) c->row_ptr[u] = gs[kg[u]];
+            for (uint64_t u = 0; u <= x->csr.U; u++) c->row_ptr[u] = gs[kg[u]];
         } else {  // segmented layout -> the compact table: bucket by bucket, keys at seg_start[b] + b + i
-            c->keys = (uint64_t*)malloc((x->U ? x->U : 1) * 8);
+            c->keys = (uint64_t*)malloc((x->csr.U ? x->csr.U : 1) * 8);
             if (!c->keys) throw std::bad_alloc();
             uint64_t u = 0;
-            for (uint32_t b = 0; b < x->seg_nb; b++) {
+            for (uint32_t b = 0; b < x->csr.seg_nb; b++) {
                 const uint64_t kb = (uint64_t)st[b] + b, tk = (uint32_t)sc[b];
-                for (uint64_t i = 0; i < tk && u < x->U; i++, u++) { c->keys[u] = keys[kb + i]; c->row_ptr[u] = gs[kg[kb + i]]; }
+                for (uint64_t i = 0; i < tk && u < x->csr.U; i++, u++) { c->keys[u] = keys[kb + i]; c->row_ptr[u] = gs[kg[kb + i]]; }
             }
-            if (u != x->U) fail(KS_ERR_CUDA, "internal error: segmented CSR does not add up");
-            c->row_ptr[x->U] = x->n_tuples;
+            if (u != x->csr.U) fail(KS_ERR_CUDA, "internal error: segmented CSR does not add up");
+            c->row_ptr[x->csr.U] = x->n_tuples;
             free(keys);
         }
         for (uint64_t i = 0; i < x->n_tuples; i++) { c->pid[i] = (uint32_t)(loc[i] >> 32); c->pos[i] = (uint32_t)loc[i]; }
@@ -1733,17 +1665,17 @@ ks_status ks_query_upload(ks_index* x, const ks_proteome* q) {
 ks_status ks_search_resident(ks_index* x, uint32_t flags, ks_search_result** out) {
     return guarded([&] {
         if (!x || !out) fail(KS_ERR_VALIDATION, "Validation error: null argument");
-        if (!x->finalized) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
         if (!x->qbatch.valid) fail(KS_ERR_VALIDATION, "Validation error: no query batch is resident");
         x->use();
         ResultDevice* rd = nullptr;
         ks_search_result* r = new_result(x, &rd);
         const bool dbg = x->hooks.timing;
-        const double t0 = dbg ? now_ms() : 0;
+        const double t0 = dbg ? wall_ms() : 0;
         try {
             const SearchOut o = search_resident_device(x, *rd->arena, (flags & KS_SEARCH_HITS) != 0,
                                                        (flags & KS_SEARCH_QUERY_SKETCHES) != 0, false, 0);
-            const double t1 = dbg ? now_ms() : 0;
+            const double t1 = dbg ? wall_ms() : 0;
             rd->block = o.block;
             rd->L = o.L;
             r->n_queries = o.L.nq;
@@ -1754,7 +1686,7 @@ ks_status ks_search_resident(ks_index* x, uint32_t flags, ks_search_result** out
             KS_CUDA(cudaEventElapsedTime(&r->ms_device, x->ev[EV_Q0], x->ev[EV_Q1]));
             x->ms_search = r->ms_device;
             if (dbg) fprintf(stderr, "[ks] search: device %.3f ms; host: kernels + count read-back %.3f ms, block read-back %.3f ms\n",
-                             r->ms_device, t1 - t0, now_ms() - t1);
+                             r->ms_device, t1 - t0, wall_ms() - t1);
         } catch (...) {
             ks_search_result_free(r);
             throw;
@@ -1856,7 +1788,7 @@ ks_status ks_shard_search_batch(ks_index* x, ks_comm* c, const ks_proteome* quer
     if (up != KS_OK) return up;
     return guarded([&] {
         if (!c || !out) fail(KS_ERR_VALIDATION, "Validation error: null argument");
-        if (!x->finalized) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
         if (c->device != x->params.device) fail(KS_ERR_VALIDATION, "Validation error: communicator and index are on different devices");
         if (pid_base + x->n_prot > 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-1 proteins over all shards");
         x->use();

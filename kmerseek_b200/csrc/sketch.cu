@@ -1044,8 +1044,6 @@ cudaError_t launch_sketch_finish(const SketchArgs& a, cudaStream_t stream) {
     return cudaMemsetAsync(a.d_count + 1, 0, 8, stream);
 }
 
-bool sketch_is_exact(const SketchArgs& a) { return exact_path(a); }
-
 cudaError_t launch_sketch(const SketchArgs& a, cudaStream_t stream, uint64_t* n_launches) {
     cudaError_t e = launch_sketch_prepare(a, stream, n_launches);
     if (e != cudaSuccess) return e;

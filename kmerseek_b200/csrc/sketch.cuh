@@ -81,7 +81,6 @@ cudaError_t launch_sketch(const SketchArgs& a, cudaStream_t stream, uint64_t* n_
 cudaError_t launch_sketch_prepare(const SketchArgs& a, cudaStream_t stream, uint64_t* n_launches);
 cudaError_t launch_sketch_tiles(const SketchArgs& a, cudaStream_t stream, uint64_t* n_launches);
 cudaError_t launch_sketch_finish(const SketchArgs& a, cudaStream_t stream);
-bool sketch_is_exact(const SketchArgs& a);
 void fill_lut(int moltype, Lut256* lut);
 // 5-bit residue codes for the packed upload format: 'A'..'Z' -> 1..26, '*' -> 27, 0 = padding.  Returns false (and
 // leaves `out` unspecified) when a byte has no code.  out must hold packed_bytes(n) bytes.
