@@ -4,6 +4,8 @@ planted queries find the protein they were cut from.  C2: 570 k proteins / 200 M
 build); C3 on one GPU: 10 000 planted domains against the same proteome, dayhoff k=16.
 And against the oracle itself on the subsamples BASELINE.md section 4 names: C2 on a 10 M-residue prefix, C3 with 1 000
 queries against a 10 M-residue prefix (hit lists bit-exact, scores within 1e-6), C4 on a 50 M-residue prefix."""
+import re
+
 import numpy as np
 import pytest
 
@@ -52,12 +54,33 @@ def _check_index(K, res, offs, k, moltype, expect_max_unique=None):
         grp_head = ~inner
         grp_head[1:] |= pid[1:] != pid[:-1]
         assert int(grp_head.sum()) == st["n_groups"]
-        return idx, st
+        return st, (keys, row_ptr, pid, pos)
 
 
-def test_c2_index_build_properties(K, proteome):
+def test_c2_index_build_properties(K, proteome, monkeypatch, capfd):
+    """... and the keys against the oracle on a seeded sample of postings: C2's dense keys need 16 + 10 + 20 + 19 = 65 bits
+    with the parity bit, so they are built without it (code = prefix << 9 | rank in the prefix group, all 64 bits)."""
+    from oracle import oracle as O
     res, offs = proteome
-    _check_index(K, res, offs, 24, "hp", expect_max_unique=1 << 24)
+    k = 24
+    assert (len(offs) - 2).bit_length() == 20 and int(np.diff(offs.astype(np.int64)).max()).bit_length() == 19
+    monkeypatch.setenv("KS_TIMING", "1")  # (read when the handle is created)
+    capfd.readouterr()
+    st, (keys, row_ptr, pid, pos) = _check_index(K, res, offs, k, "hp", expect_max_unique=1 << 24)
+    err = capfd.readouterr().err
+    begin = re.search(r"^\[ks\] dense begin: state 1 rb (\d+)$", err, re.M)
+    fin = re.search(r"^\[ks\] dense finalize: .* unhandled 0 .* rb (\d+)$", err, re.M)
+    assert begin and fin and (int(begin.group(1)), int(fin.group(1))) == (10, 9), err  # no parity bit
+    assert st["build_path"] == 1
+    # the key of a posting's row is the hash of the posting's window: the sampled windows, one per protein, to the oracle
+    j = np.random.default_rng(20260109).integers(0, len(pid), size=4096)
+    row = np.searchsorted(row_ptr, j, "right") - 1
+    start = offs[:-1].astype(np.int64)[pid[j]] + pos[j].astype(np.int64)
+    wres = res[start[:, None] + np.arange(k)].ravel()
+    woffs = np.arange(0, k * len(j) + 1, k, dtype=np.uint64)
+    oh, opid, opos = O.sketch_tuples(wres, woffs, k, "hp", 1)
+    assert np.array_equal(opid, np.arange(len(j))) and not opos.any()
+    assert np.array_equal(keys[row], oh)
 
 
 def test_c3_planted_queries_find_their_source(K, proteome):

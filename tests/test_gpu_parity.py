@@ -552,24 +552,28 @@ def test_bucket_sort_path_scaled(K, O):
         assert np.array_equal(pid, ops) and np.array_equal(pos, oqs)
 
 
-def _csr_equals_oracle(K, O, res, offs, k, moltype, scaled=1, path=None):
-    prot = K.Proteome.from_packed(res, offs)
-    with K.ProteomeIndex("db", k, scaled, moltype) as idx:
-        idx.add_proteome(prot)
-        idx.finalize()
-        keys, row_ptr, pid, pos = idx.csr()
-        oh, opid, opos = O.sketch_tuples(res, offs, k, moltype, scaled)
-        okeys, orow, ops, oqs = O.build_index(oh, opid, opos)
-        assert np.array_equal(keys, okeys) and np.array_equal(row_ptr, orow), (k, moltype)
-        assert np.array_equal(pid, ops) and np.array_equal(pos, oqs), (k, moltype)
-        st = idx.stats()
-        assert st["n_tuples"] == len(oh) and st["n_unique_hashes"] == len(okeys)
-        assert path is None or st["build_path"] == path, (st["build_path"], path)
-        sk = idx.export_sketches()
-        osk = O.protein_sketches(oh, opid, len(offs) - 1)
-        for (m, a), (om, oa) in zip(sk, osk):
-            assert np.array_equal(m, om) and np.array_equal(a, oa)
-        return st
+def _csr_equals_oracle(K, O, res, offs, k, moltype, scaled=1, path=None, idx=None):
+    """idx: a handle that (res, offs) has been added to; a new one takes them otherwise."""
+    if idx is None:
+        prot = K.Proteome.from_packed(res, offs)
+        with K.ProteomeIndex("db", k, scaled, moltype) as idx:
+            idx.add_proteome(prot)
+            return _csr_equals_oracle(K, O, res, offs, k, moltype, scaled, path, idx)
+    idx.finalize()
+    keys, row_ptr, pid, pos = idx.csr()
+    oh, opid, opos = O.sketch_tuples(res, offs, k, moltype, scaled)
+    okeys, orow, ops, oqs = O.build_index(oh, opid, opos)
+    assert np.array_equal(keys, okeys) and np.array_equal(row_ptr, orow), (k, moltype)
+    assert np.array_equal(pid, ops) and np.array_equal(pos, oqs), (k, moltype)
+    st = idx.stats()
+    assert st["n_tuples"] == len(oh) and st["n_unique_hashes"] == len(okeys)
+    assert path is None or st["build_path"] == path, (st["build_path"], path)
+    sk = idx.export_sketches()
+    osk = O.protein_sketches(oh, opid, len(offs) - 1)
+    assert len(sk) == len(osk)
+    for (m, a), (om, oa) in zip(sk, osk):
+        assert np.array_equal(m, om) and np.array_equal(a, oa)
+    return st
 
 
 def test_dense_kmer_space_path(K, O, monkeypatch):
