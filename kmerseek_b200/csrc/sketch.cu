@@ -1,24 +1,30 @@
-// Fused sketch kernel for sm_100a.
+// Sketch stage for sm_100a.
 //
-// One launch does, for every k-mer window of every protein of the resident batch:
+// For every k-mer window of every protein of the resident batch:
 //   reduced-alphabet translation (256-entry LUT in shared memory)        -- src/rust/encoding.rs:43-53
 //   MurmurHash3_x64_128(translated k-mer, seed 42), low word            -- sourmash::_hash_murmur, src/rust/index.rs:766
 //   FracMinHash filter  h != 0 && h <= max_hash                          -- KmerMinHash::add_protein, src/rust/signature.rs:273-274
-//   ordered compaction of the surviving (hash, protein, pos) tuples      -- process_kmers, src/rust/index.rs:749-786
+//   output of the surviving (hash, protein, pos) tuples                  -- process_kmers, src/rust/index.rs:749-786
 // (paths relative to the reference repository).  Data layout and roofline: DESIGN.md section 3.
 //
-// Shape: the residue stream is cut into tiles of SK_TILE window-start positions.  A CTA takes a tile
-// (dynamic ticket, so a tile's predecessors have always started), pulls SK_TILE + k - 1 residues with
-// coalesced 16-byte loads, translates them once into shared memory, and each warp then walks 8 rows of
-// 32 consecutive windows: lane l of row r owns window (warp*8 + r)*32 + l, rebuilds its k bytes from
-// aligned shared-memory words with funnel shifts, hashes in registers, and the row is compacted with a
-// ballot into a per-warp staging area (conflict-free, lanes write consecutive slots).  Tile totals are
-// chained across CTAs with a single-pass decoupled look-back, after which every warp streams its staged
-// tuples to their final, globally ordered position with fully coalesced stores.  Output order is
-// (protein, pos), independent of scheduling, so the later stable sort by hash is deterministic.
+// Three kernels: sketch_quad_kernel (k <= 32: every lane hashes 4 consecutive windows), sketch_dense_kernel (hp,
+// 8 <= k <= 24: a window's hash is a table entry and its tuple one 64-bit key) and sketch_kernel (k > 32: a byte loop per
+// window).  All three cut the residue stream into tiles of SK_TILE window starts, one tile per CTA, and are built from
+// the same parts: the tile's residues staged once, translated, in shared memory (stage_residues); the offsets of the
+// proteins that intersect the tile (cache_offsets) and every lane's forward walk over them (first_protein,
+// seek_protein); and the ordered output (warp_prefix, exact_base / lookback_base, write_warp).
+//
+// Ordered output is in (protein, pos) order, independent of scheduling, so the later stable sort by hash is
+// deterministic: each row of windows is ranked with ballots into a per-warp staging area in shared memory, and every
+// warp streams its staged entries to their final position with coalesced stores.  The tile's base is known up front on
+// the exact path (scaled == 1: tile_count_kernel + scan, no cross-CTA dependency); otherwise CTAs take tiles by ticket
+// (a tile's predecessors have always started) and chain the tile totals with a single-pass decoupled look-back.
+// Unordered output (the quad kernel's SCATTER, the dense kernel's scatter) keeps the keys in registers and hands them
+// straight to the first level of the partition (dense_scatter.cuh): no ranking and no staging in window order.
 #include <cub/device/device_scan.cuh>
 
 #include <cstring>
+#include <type_traits>
 
 #include "common.cuh"
 #include "sketch.cuh"
@@ -28,40 +34,6 @@ namespace ks {
 namespace {
 
 constexpr int OFFS_CACHE = 256;  // offsets of the proteins that intersect a tile, cached in smem when they fit
-
-template <int K>
-__device__ __forceinline__ uint64_t murmur_words(const uint32_t* a) {
-    // a[] = the K translated bytes, little-endian packed, bytes past K zeroed.
-    constexpr int NB = K / 16, REM = K % 16, NWORDS = (K + 3) / 4;
-    uint64_t h1 = SEED, h2 = SEED;
-#pragma unroll
-    for (int b = 0; b < NB; b++) {
-        uint64_t k1 = (uint64_t)a[4 * b] | ((uint64_t)a[4 * b + 1] << 32);
-        uint64_t k2 = (uint64_t)a[4 * b + 2] | ((uint64_t)a[4 * b + 3] << 32);
-        h1 ^= mix_k1(k1);
-        h1 = rotl64(h1, 27) + h2;
-        h1 = h1 * 5 + 0x52dce729;
-        h2 ^= mix_k2(k2);
-        h2 = rotl64(h2, 31) + h1;
-        h2 = h2 * 5 + 0x38495ab5;
-    }
-    auto word = [&](int i) -> uint64_t { return i < NWORDS ? (uint64_t)a[i] : 0ull; };
-    if (REM > 8) {
-        uint64_t k2 = word(4 * NB + 2) | (word(4 * NB + 3) << 32);
-        h2 ^= mix_k2(k2);
-    }
-    if (REM > 0) {
-        uint64_t k1 = word(4 * NB) | (word(4 * NB + 1) << 32);
-        h1 ^= mix_k1(k1);
-    }
-    h1 ^= (uint64_t)K;
-    h2 ^= (uint64_t)K;
-    h1 += h2;
-    h2 += h1;
-    h1 = fmix64(h1);
-    h2 = fmix64(h2);
-    return h1 + h2;
-}
 
 struct Workspace {
     uint32_t* ticket;      // [0] tile ticket, [1] zero-hash flag (exact path)
@@ -131,12 +103,180 @@ __global__ void tile_count_kernel(const uint64_t* __restrict__ offsets, uint64_t
     tile_cnt[t] = c;
 }
 
-template <int K, bool TRANSLATE>
+// ---------------------------------------------------------------------------------------------
+// Parts shared by the kernels
+// ---------------------------------------------------------------------------------------------
+constexpr int WARP_SLOTS = SK_TILE / (SK_THREADS / 32);  // staging slots per warp (256): one per window of the warp
+
+// Entry c of the code table of the packed residue format (pack_residues: 'A'..'Z' -> 1..26, '*' -> 27), translated.
+__device__ __forceinline__ uint8_t lut32_entry(const uint8_t* lut, uint32_t c) {
+    return c == 0 ? 0 : c <= 26 ? lut['A' + c - 1] : c == 27 ? lut['*'] : 0;
+}
+
+// Residues [g0, g0 + n) of the batch into s_res as translated bytes (n + 15 bytes of room).  Packed residues: thread t
+// unpacks the 5-bit groups t, t + SK_THREADS, ... (8 residues = 5 bytes) through s_lut32, which the caller has filled.
+// Plain residues: coalesced 16-byte loads, translated through s_lut when TRANSLATE, 16-byte shared stores (n <= 16 *
+// SK_THREADS).  Groups and chunks that start past the batch are not backed by memory and stage zeros.  The caller puts a
+// barrier between this and the first read of s_res.
+template <bool TRANSLATE>
+__device__ __forceinline__ void stage_residues(uint32_t tid, uint32_t* s_res, const SketchArgs& a, bool packed, uint64_t g0,
+                                               uint32_t n, const uint8_t* s_lut, const uint8_t* s_lut32) {
+    if (packed) {
+        const uint32_t n_groups = (n + 7) / 8;
+        for (uint32_t grp = tid; grp < n_groups; grp += SK_THREADS) {
+            const uint64_t group = g0 / 8 + grp;
+            const uint64_t byte = group * 5;
+            uint32_t w0 = 0, w1 = 0;
+            if (group * 8 < a.n_res) {
+                const uint32_t* w = reinterpret_cast<const uint32_t*>(a.residues + (byte & ~3ull));
+                w0 = __ldg(w);
+                w1 = __ldg(w + 1);
+            }
+            const uint32_t sh8 = (uint32_t)(byte & 3) * 8;
+            const uint32_t lo = __funnelshift_r(w0, w1, sh8), hi = (w1 >> sh8) & 0xffu;  // 40 bits: lo | hi << 32
+            uint32_t o0 = 0, o1 = 0;
+#pragma unroll
+            for (int i = 0; i < 4; i++) o0 |= (uint32_t)s_lut32[(lo >> (5 * i)) & 31u] << (8 * i);
+            o1 |= (uint32_t)s_lut32[(lo >> 20) & 31u];
+            o1 |= (uint32_t)s_lut32[(lo >> 25) & 31u] << 8;
+            o1 |= (uint32_t)s_lut32[((lo >> 30) | (hi << 2)) & 31u] << 16;
+            o1 |= (uint32_t)s_lut32[(hi >> 3) & 31u] << 24;
+            s_res[2 * grp] = o0;
+            s_res[2 * grp + 1] = o1;
+        }
+    } else {
+        const uint32_t n_chunks = (n + 15) / 16;
+        if (tid < n_chunks) {
+            const uint64_t g = g0 + 16ull * tid;
+            uint4 v = make_uint4(0, 0, 0, 0);
+            if (g < a.n_res) v = __ldg(reinterpret_cast<const uint4*>(a.residues + g));
+            if (TRANSLATE) {
+                uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                for (int i = 0; i < 4; i++) {
+                    const uint32_t x = w[i];
+                    w[i] = (uint32_t)s_lut[x & 0xff] | ((uint32_t)s_lut[(x >> 8) & 0xff] << 8) |
+                           ((uint32_t)s_lut[(x >> 16) & 0xff] << 16) | ((uint32_t)s_lut[x >> 24] << 24);
+                }
+                v = make_uint4(w[0], w[1], w[2], w[3]);
+            }
+            reinterpret_cast<uint4*>(s_res)[tid] = v;
+        }
+    }
+}
+
+// The proteins that intersect a tile are [p_lo, p_hi] = tile_pid[tile], tile_pid[tile + 1].  Caches their offsets,
+// offsets[p_lo .. p_hi + 1], in s_offs when they fit; returns whether they do.  A barrier must follow before the first
+// lookup.
+__device__ __forceinline__ bool cache_offsets(uint32_t tid, const SketchArgs& a, uint64_t* s_offs, uint32_t p_lo, uint32_t p_hi) {
+    const uint32_t n_off = p_hi - p_lo + 2;
+    const bool cached = n_off <= OFFS_CACHE;
+    if (cached)
+        for (uint32_t i = tid; i < n_off; i += SK_THREADS) s_offs[i] = a.offsets[p_lo + i];
+    return cached;
+}
+
+// Residues from the tile start g0 on, clamped (window w of the tile exists iff w < the result).
+__device__ __forceinline__ uint32_t tile_residues(const SketchArgs& a, uint64_t g0) {
+    const uint64_t left = a.n_res - g0;
+    return left > 0x40000000ull ? 0x40000000u : (uint32_t)left;
+}
+
+// A lane's walk over the proteins of its tile.  Windows are named by their start w relative to the tile start g0, and
+// a lane's windows only move forward.  The state is the lane's protein p, its start as the low 32 bits of the absolute
+// position (positions within a protein fit 32 bits) and its end relative to the tile start, clamped so that 32-bit
+// compares suffice (end_rel).  offs: offsets[], from the shared-memory cache when the tile's slice is there.
+__device__ __forceinline__ uint32_t end_rel(uint64_t o, uint64_t g0) {
+    const uint64_t d = o - g0;
+    return d > 0x7fffffffull ? 0x7fffffffu : (uint32_t)d;
+}
+// the protein of window w (which exists): binary search over the tile's proteins [p_lo, p_hi]
+__device__ __forceinline__ void first_protein(const uint64_t* offs, uint64_t g0, uint32_t p_lo, uint32_t p_hi, uint32_t w,
+                                              uint32_t& p, uint32_t& pstart_lo, uint32_t& pend_rel) {
+    const uint64_t g = g0 + w;
+    uint32_t lo = p_lo, hi = p_hi;
+    while (lo < hi) {
+        const uint32_t mid = (lo + hi + 1) >> 1;
+        if (offs[mid] <= g) lo = mid; else hi = mid - 1;
+    }
+    p = lo;
+    pstart_lo = (uint32_t)offs[p];
+    pend_rel = end_rel(offs[p + 1], g0);
+}
+// forward to the protein of window w (which exists and is not before the lane's current window)
+__device__ __forceinline__ void seek_protein(const uint64_t* offs, uint64_t g0, uint32_t w, uint32_t& p, uint32_t& pstart_lo,
+                                             uint32_t& pend_rel) {
+    while (w >= pend_rel) { p++; pstart_lo = (uint32_t)offs[p]; pend_rel = end_rel(offs[p + 1], g0); }
+}
+
+// Ordered output, after every warp has staged its wcount entries: the warps' prefix over the staged counts (contains a
+// barrier).  wprefix = entries of the warps before this one, btotal = entries of the tile.
+struct WarpPrefix { uint32_t wprefix, btotal; };
+__device__ __forceinline__ WarpPrefix warp_prefix(uint32_t tid, uint32_t* s_wtot, uint32_t wcount) {
+    const uint32_t lane = tid & 31, warp = tid >> 5;
+    if (lane == 0) s_wtot[warp] = wcount;
+    __syncthreads();
+    WarpPrefix r{0, 0};
+#pragma unroll
+    for (int i = 0; i < SK_THREADS / 32; i++) {
+        const uint32_t t = s_wtot[i];
+        if (i < (int)warp) r.wprefix += t;
+        r.btotal += t;
+    }
+    return r;
+}
+
+// Output position of the tile's first entry, exact path: the tile's base from tile_count_kernel + scan.  The last tile
+// sets d_count[0].
+__device__ __forceinline__ uint64_t exact_base(uint32_t tid, const SketchArgs& a, uint32_t tile, const uint64_t* tile_base,
+                                               uint32_t btotal) {
+    const uint64_t base = tile_base[tile];
+    if (tid == 0 && tile == n_tiles_of(a.n_res) - 1) *a.d_count = base + btotal;
+    return base;
+}
+
+// The same on the look-back path: warp 0 chains the tile's total behind its predecessors' (contains a barrier).
+__device__ __forceinline__ uint64_t lookback_base(uint32_t lane, uint32_t warp, const SketchArgs& a, uint32_t tile,
+                                                  uint64_t* status, uint32_t btotal, uint64_t& s_base) {
+    if (warp == 0) {
+        const uint64_t excl = scan_lookback(status, tile, btotal);
+        if (lane == 0) {
+            s_base = excl;
+            if (tile == n_tiles_of(a.n_res) - 1) *a.d_count = excl + btotal;
+        }
+    }
+    __syncthreads();
+    return s_base;
+}
+
+// A warp's share of the ordered output: its staged entries 0 .. wcount - 1 go to output positions base + i.  Positions
+// at or past a.capacity are not written (the caller sees the full count in d_count and retries with room).  put(i)
+// writes entry i.
+template <class Put>
+__device__ __forceinline__ void write_warp(uint32_t lane, const SketchArgs& a, uint64_t base, uint32_t wcount, Put put) {
+    if (base + wcount <= a.capacity) {  // the usual case: the warp's 256 slots, 8 per lane, no per-element bound check
+#pragma unroll
+        for (uint32_t i0 = 0; i0 < WARP_SLOTS; i0 += 32) {
+            const uint32_t i = i0 + lane;
+            if (i0 >= wcount) break;  // uniform
+            if (i < wcount) put(i);
+        }
+    } else {
+        for (uint32_t i = lane; i < wcount; i += 32)
+            if (base + i < a.capacity) put(i);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Byte-loop kernel (k > 32): lane l of row r owns window (warp * SK_ROWS + r) * 32 + l and hashes its k bytes straight
+// from shared memory; a row is compacted with one ballot (lanes write consecutive slots).  Ordered output on the
+// look-back path only (exact_path and the scatter route take k <= 32).
+// ---------------------------------------------------------------------------------------------
+template <bool TRANSLATE>
 __global__ void __launch_bounds__(SK_THREADS)
 sketch_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint64_t* __restrict__ status,
               const uint32_t* __restrict__ tile_pid) {
-    constexpr int KMAX = K == 0 ? SK_MAX_K : K;
-    constexpr int RES_WORDS = (SK_TILE + KMAX + 16 + 3) / 4;
+    constexpr int RES_WORDS = (SK_TILE + SK_MAX_K + 16 + 3) / 4;
     __shared__ __align__(16) uint32_t s_res[RES_WORDS];
     __shared__ __align__(16) uint64_t s_hash[SK_TILE];
     __shared__ __align__(16) uint64_t s_loc[SK_TILE];
@@ -147,123 +287,51 @@ sketch_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint64_t*
     __shared__ uint64_t s_base;
 
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t k = K == 0 ? a.k : (uint32_t)K;
+    const uint32_t k = a.k;
 
     if (tid == 0) s_tile = atomicAdd(ticket, 1u);
     if (TRANSLATE) s_lut[tid] = lut.b[tid];
     __syncthreads();
     const uint32_t tile = s_tile;
     const uint64_t g0 = (uint64_t)tile * SK_TILE;
-    const uint64_t n_tiles = n_tiles_of(a.n_res);
-
-    // proteins that intersect this tile: [p_lo, p_hi]; cache offsets[p_lo .. p_hi+1]
     const uint32_t p_lo = tile_pid[tile], p_hi = tile_pid[tile + 1];
-    const uint32_t n_off = p_hi - p_lo + 2;
-    const bool cached = n_off <= OFFS_CACHE;
-    if (cached)
-        for (uint32_t i = tid; i < n_off; i += SK_THREADS) s_offs[i] = a.offsets[p_lo + i];
-
-    // stage residues: coalesced 16-byte loads, translate once, 16-byte shared stores
-    {
-        const uint32_t n_chunks = (SK_TILE + k - 1 + 15) / 16;
-        if (tid < n_chunks) {
-            uint64_t g = g0 + 16ull * tid;
-            uint4 v = make_uint4(0, 0, 0, 0);
-            if (g < a.n_res) v = __ldg(reinterpret_cast<const uint4*>(a.residues + g));
-            if (TRANSLATE) {
-                uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    uint32_t x = w[i];
-                    w[i] = (uint32_t)s_lut[x & 0xff] | ((uint32_t)s_lut[(x >> 8) & 0xff] << 8) |
-                           ((uint32_t)s_lut[(x >> 16) & 0xff] << 16) | ((uint32_t)s_lut[x >> 24] << 24);
-                }
-                v = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-            reinterpret_cast<uint4*>(s_res)[tid] = v;
-        }
-    }
+    const bool cached = cache_offsets(tid, a, s_offs, p_lo, p_hi);
+    stage_residues<TRANSLATE>(tid, s_res, a, false, g0, SK_TILE + k - 1, s_lut, nullptr);  // (k > 32 is never uploaded packed)
     __syncthreads();
 
     const uint64_t* offs = cached ? (const uint64_t*)s_offs - p_lo : a.offsets;
-
-    // protein of this lane's first window
-    const uint32_t w0 = warp * (SK_ROWS * 32) + lane;  // tile-local index of row 0's window
-    uint64_t g = g0 + w0;
-    uint32_t p = p_lo;
-    uint64_t pstart = 0, pend = 0;
-    if (g < a.n_res) {
-        uint32_t lo = p_lo, hi = p_hi;
-        while (lo < hi) {
-            uint32_t mid = (lo + hi + 1) >> 1;
-            if (offs[mid] <= g) lo = mid; else hi = mid - 1;
-        }
-        p = lo;
-        pstart = offs[p];
-        pend = offs[p + 1];
-    }
+    const uint32_t nres_rel = tile_residues(a, g0), g0_lo = (uint32_t)g0;
+    const uint32_t w0 = warp * WARP_SLOTS + lane;  // the lane's window in row 0
+    uint32_t p = p_lo, pstart_lo = 0, pend_rel = 0;
+    if (w0 < nres_rel) first_protein(offs, g0, p_lo, p_hi, w0, p, pstart_lo, pend_rel);
 
     uint32_t wcount = 0;  // tuples staged by this warp so far (uniform across the warp)
-    const uint32_t sh = (lane & 3) * 8;
 #pragma unroll
-    for (int r = 0; r < SK_ROWS; r++, g += 32) {
-        const uint32_t wi = w0 + r * 32;
+    for (int r = 0; r < SK_ROWS; r++) {
+        const uint32_t w = w0 + r * 32;
         bool valid = false;
-        if (g < a.n_res) {
-            while (g >= pend) { p++; pstart = pend; pend = offs[p + 1]; }
-            valid = g + k <= pend;
+        if (w < nres_rel) {
+            seek_protein(offs, g0, w, p, pstart_lo, pend_rel);
+            valid = w + k <= pend_rel;
         }
-        uint64_t h;
-        if (K == 0) {
-            h = valid ? murmur_bytes(reinterpret_cast<const uint8_t*>(s_res) + wi, k) : 0;
-        } else {
-            constexpr int NW = (KMAX + 3 + 3) / 4;  // aligned words that cover bytes [wi, wi+K)
-            constexpr int KW = (KMAX + 3) / 4;
-            uint32_t x[NW + 1];
-#pragma unroll
-            for (int i = 0; i < NW; i++) x[i] = s_res[(wi >> 2) + i];
-            x[NW] = 0;
-            uint32_t b[KW];
-#pragma unroll
-            for (int i = 0; i < KW; i++) b[i] = __funnelshift_r(x[i], x[i + 1], sh);
-            if (KMAX % 4) b[KW - 1] &= (1u << (8 * (KMAX % 4))) - 1u;
-            h = murmur_words<KMAX>(b);
-        }
+        const uint64_t h = valid ? murmur_bytes(reinterpret_cast<const uint8_t*>(s_res) + w, k) : 0;
         const bool keep = valid && h != 0 && h <= a.max_hash;
         const uint32_t bal = __ballot_sync(0xffffffffu, keep);
         if (keep) {
-            const uint32_t slot = warp * (SK_ROWS * 32) + wcount + __popc(bal & ((1u << lane) - 1u));
+            const uint32_t slot = warp * WARP_SLOTS + wcount + __popc(bal & ((1u << lane) - 1u));
             s_hash[slot] = h;
-            s_loc[slot] = ((uint64_t)(a.pid_base + p) << 32) | (uint64_t)(uint32_t)(g - pstart);
+            s_loc[slot] = ((uint64_t)(a.pid_base + p) << 32) | (uint64_t)(g0_lo + w - pstart_lo);
         }
         wcount += __popc(bal);
     }
 
-    if (lane == 0) s_wtot[warp] = wcount;
-    __syncthreads();
-    uint32_t wprefix = 0, btotal = 0;
-#pragma unroll
-    for (int i = 0; i < SK_THREADS / 32; i++) {
-        uint32_t t = s_wtot[i];
-        if (i < (int)warp) wprefix += t;
-        btotal += t;
-    }
-    if (warp == 0) {
-        uint64_t excl = scan_lookback(status, tile, btotal);
-        if (lane == 0) {
-            s_base = excl;
-            if (tile == n_tiles - 1) *a.d_count = excl + btotal;
-        }
-    }
-    __syncthreads();
-    const uint64_t base = s_base + wprefix;
-    const uint32_t sbase = warp * (SK_ROWS * 32);
-    for (uint32_t i = lane; i < wcount; i += 32) {
-        if (base + i < a.capacity) {
-            a.out_hash[base + i] = s_hash[sbase + i];
-            a.out_loc[base + i] = s_loc[sbase + i];
-        }
-    }
+    const WarpPrefix wp = warp_prefix(tid, s_wtot, wcount);
+    const uint64_t base = lookback_base(lane, warp, a, tile, status, wp.btotal, s_base) + wp.wprefix;
+    const uint32_t sbase = warp * WARP_SLOTS;
+    write_warp(lane, a, base, wcount, [&](uint32_t i) {
+        a.out_hash[base + i] = s_hash[sbase + i];
+        a.out_loc[base + i] = s_loc[sbase + i];
+    });
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -273,8 +341,8 @@ sketch_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint64_t*
 // and each window is cut out with constant funnel shifts.  MurmurHash3 runs on explicit 32-bit limbs so that a
 // 64-bit multiply by a constant is three IMADs and a 64-bit rotate two SHFs (left to the compiler, the same
 // arithmetic took about twice the instructions, and the kernel is issue-bound before it is HBM-bound).
-// Positions are tile-relative 32-bit values.  Kept tuples are staged in shared memory at their ordered slot;
-// the slot -> address map interleaves the four windows of a quad over four segments so that both the quad
+// Positions are tile-relative 32-bit values.  Ordered output stages kept tuples in shared memory at their ordered
+// slot; the slot -> address map interleaves the four windows of a quad over four segments so that both the quad
 // writes and the linear read-out are bank-conflict free.
 // ---------------------------------------------------------------------------------------------
 struct L64 { uint32_t lo, hi; };
@@ -340,33 +408,77 @@ __device__ __forceinline__ uint64_t murmur_limbs(const uint32_t* a) {
 constexpr int SQ_ROWS = SK_TILE / (SK_THREADS * 4);   // quad rows per warp (2)
 constexpr int SQ_SEG = SK_TILE / 4 + 4;                // staging segment stride in slots: = 4 (mod 16)
 __device__ __forceinline__ uint32_t stage_addr(uint32_t slot) { return (slot & 3u) * SQ_SEG + (slot >> 2); }
+static_assert(DS_ITEMS == SQ_ROWS * 4, "a thread's windows are its scatter items");
+static_assert(DS_THREADS == SK_THREADS && DS_TILE == SK_TILE, "one scatter tile per sketch tile");
 
-// FULL (max_hash = 2^64 - 1, i.e. scaled == 1): tile bases come from tile_count_kernel + scan, so there is no
-// ticket, no look-back chain and no cross-CTA dependency at all.
-#ifndef KS_DIRECT_SCATTER
-#define KS_DIRECT_SCATTER 1  // unordered output: keys go from registers straight into the scatter (no ranking, no staging in order)
-#endif
-template <int K, bool TRANSLATE, bool FULL, bool SCATTER>
+// The bytes of quad q (windows 4q .. 4q + 3 of the tile): the aligned words of s_res that cover them.
+template <int K>
+struct Quad {
+    static constexpr int NW = (K + 3 + 3) / 4;  // words that cover the 4 + K - 1 bytes of a quad
+    static constexpr int KW = (K + 3) / 4;      // words of one window
+    uint32_t x[NW + 1];
+    __device__ __forceinline__ Quad(const uint32_t* s_res, uint32_t q) {
+#pragma unroll
+        for (int i = 0; i < NW; i++) x[i] = s_res[q + i];
+        x[NW] = 0;
+    }
+    // MurmurHash3 of window j of the quad: its K bytes cut out with a funnel shift, bytes past K zeroed
+    __device__ __forceinline__ uint64_t hash(int j) const {
+        uint32_t b[KW];
+#pragma unroll
+        for (int i = 0; i < KW; i++) b[i] = j == 0 ? x[i] : __funnelshift_r(x[i], x[i + 1], 8 * j);
+        if (K % 4) b[KW - 1] &= (1u << (8 * (K % 4))) - 1u;
+        return murmur_limbs<K>(b);
+    }
+};
+
+// Ordered staging of one quad row: the kept windows of the warp's 32 quads are ranked in window order (lane, then j) with
+// four ballots, and put(j, addr) stores this lane's window j at its staging address.  wcount: entries the warp has
+// staged so far (uniform across the warp).
+template <class Put>
+__device__ __forceinline__ void stage_row(uint32_t lane, uint32_t warp, const bool (&keep)[4], uint32_t& wcount, Put put) {
+    const uint32_t lt = (1u << lane) - 1u;
+    uint32_t below = 0, total = 0;
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        const uint32_t bal = __ballot_sync(0xffffffffu, keep[j]);
+        below += __popc(bal & lt);
+        total += __popc(bal);
+    }
+    uint32_t slot = warp * WARP_SLOTS + wcount + below;
+#pragma unroll
+    for (int j = 0; j < 4; j++) {
+        if (keep[j]) {
+            put(j, stage_addr(slot));
+            slot++;
+        }
+    }
+    wcount += total;
+}
+
 #ifndef KS_SK_CTAS
 #define KS_SK_CTAS 5
 #endif
 #ifndef KS_SK_CTAS_LB
 #define KS_SK_CTAS_LB 6
 #endif
+// FULL (max_hash = 2^64 - 1, i.e. scaled == 1): tile bases come from tile_count_kernel + scan, so there is no ticket, no
+// look-back chain and no cross-CTA dependency at all.  SCATTER: unordered output, the first level of the partition
+// follows in this kernel; hashes stay in registers and a window's loc waits in its own staging slot.
 // CTAs per SM the register allocation aims at (FULL: exact path / look-back path).  Measured (round 2, C4 slice, the
 // look-back path): 4 / 5 / 6 CTAs 9.26 / 7.75 / 6.77 ms (left to the compiler the non-scatter instantiations took 62-64
 // registers = 4 CTAs); the exact path is best at 5 (100 M-residue target run 0.90 ms against 0.97 ms at 6).
+template <int K, bool TRANSLATE, bool FULL, bool SCATTER>
 __global__ void __launch_bounds__(SK_THREADS, FULL ? KS_SK_CTAS : KS_SK_CTAS_LB)
 sketch_quad_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint64_t* __restrict__ status,
                    const uint32_t* __restrict__ tile_pid, const uint64_t* __restrict__ tile_base) {
     constexpr int RES_WORDS = (SK_TILE + K + 16 + 3) / 4;
-    constexpr int NW = (K + 3 + 3) / 4;  // words that cover the 4 + K - 1 bytes of a quad
-    constexpr int KW = (K + 3) / 4;
     __shared__ __align__(16) uint32_t s_res[RES_WORDS];
     __shared__ __align__(16) uint64_t s_hash[4 * SQ_SEG];
     __shared__ __align__(16) uint64_t s_loc[4 * SQ_SEG];
     __shared__ uint64_t s_offs[OFFS_CACHE];
     __shared__ uint8_t s_lut[256];
+    __shared__ uint8_t s_lut32[32];
     __shared__ uint32_t s_wtot[SK_THREADS / 32];
     __shared__ uint32_t s_tile;
     __shared__ uint64_t s_base;
@@ -380,102 +492,31 @@ sketch_quad_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint
     if (!FULL || TRANSLATE) __syncthreads();
     const uint32_t tile = FULL ? blockIdx.x + a.tile_begin : s_tile;
     const uint64_t g0 = (uint64_t)tile * SK_TILE;
-    const uint64_t n_tiles = n_tiles_of(a.n_res);
     const uint32_t p_lo = tile_pid[tile], p_hi = tile_pid[tile + 1];
-    const uint32_t n_off = p_hi - p_lo + 2;
-    const bool cached = n_off <= OFFS_CACHE;
-    if (cached)
-        for (uint32_t i = tid; i < n_off; i += SK_THREADS) s_offs[i] = a.offsets[p_lo + i];
-    if (a.packed) {
-        // 5-bit packed residues: thread g unpacks group g (8 residues = 5 bytes) through a 32-entry code table
-        __shared__ uint8_t s_lut32[32];
-        if (tid < 32) {
-            const uint32_t c = tid;
-            s_lut32[c] = c == 0 ? 0 : c <= 26 ? lut.b['A' + c - 1] : c == 27 ? lut.b['*'] : 0;
-        }
+    const bool cached = cache_offsets(tid, a, s_offs, p_lo, p_hi);
+    if (a.packed) {  // (the code table is filled here, behind its own barrier, only when it is used)
+        if (tid < 32) s_lut32[tid] = lut32_entry(lut.b, tid);
         __syncthreads();
-        constexpr uint32_t n_groups = (SK_TILE + K - 1 + 7) / 8;
-        for (uint32_t grp = tid; grp < n_groups; grp += SK_THREADS) {
-            const uint64_t group = g0 / 8 + grp;
-            const uint64_t byte = group * 5;
-            uint32_t w0 = 0, w1 = 0;
-            if (group * 8 < a.n_res) {  // groups past the last residue are not backed by memory
-                const uint32_t* w = reinterpret_cast<const uint32_t*>(a.residues + (byte & ~3ull));
-                w0 = __ldg(w);
-                w1 = __ldg(w + 1);
-            }
-            const uint32_t sh8 = (uint32_t)(byte & 3) * 8;
-            const uint32_t lo = __funnelshift_r(w0, w1, sh8), hi = (w1 >> sh8) & 0xffu;  // 40 bits: lo | hi << 32
-            uint32_t o0 = 0, o1 = 0;
-#pragma unroll
-            for (int i = 0; i < 4; i++) o0 |= (uint32_t)s_lut32[(lo >> (5 * i)) & 31u] << (8 * i);
-            o1 |= (uint32_t)s_lut32[(lo >> 20) & 31u];
-            o1 |= (uint32_t)s_lut32[(lo >> 25) & 31u] << 8;
-            o1 |= (uint32_t)s_lut32[((lo >> 30) | (hi << 2)) & 31u] << 16;
-            o1 |= (uint32_t)s_lut32[(hi >> 3) & 31u] << 24;
-            s_res[2 * grp] = o0;
-            s_res[2 * grp + 1] = o1;
-        }
+        stage_residues<TRANSLATE>(tid, s_res, a, true, g0, SK_TILE + K - 1, s_lut, s_lut32);
     } else {
-        constexpr uint32_t n_chunks = (SK_TILE + K - 1 + 15) / 16;
-        if (tid < n_chunks) {
-            const uint64_t g = g0 + 16ull * tid;
-            uint4 v = make_uint4(0, 0, 0, 0);
-            if (g < a.n_res) v = __ldg(reinterpret_cast<const uint4*>(a.residues + g));
-            if (TRANSLATE) {
-                uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-                for (int i = 0; i < 4; i++) {
-                    const uint32_t x = w[i];
-                    w[i] = (uint32_t)s_lut[x & 0xff] | ((uint32_t)s_lut[(x >> 8) & 0xff] << 8) |
-                           ((uint32_t)s_lut[(x >> 16) & 0xff] << 16) | ((uint32_t)s_lut[x >> 24] << 24);
-                }
-                v = make_uint4(w[0], w[1], w[2], w[3]);
-            }
-            reinterpret_cast<uint4*>(s_res)[tid] = v;
-        }
+        stage_residues<TRANSLATE>(tid, s_res, a, false, g0, SK_TILE + K - 1, s_lut, s_lut32);
     }
     __syncthreads();
 
     const uint64_t* offs = cached ? (const uint64_t*)s_offs - p_lo : a.offsets;
-    const uint64_t left = a.n_res - g0;
-    const uint32_t nres_rel = left > 0x40000000ull ? 0x40000000u : (uint32_t)left;  // residues from the tile start on
-    auto rel = [&](uint64_t o) -> uint32_t {  // protein end, relative to the tile start, clamped
-        const uint64_t d = o - g0;
-        return d > 0x7fffffffull ? 0x7fffffffu : (uint32_t)d;
-    };
-
-    uint32_t p = p_lo, pstart_lo = 0, pend_rel = 0;
+    const uint32_t nres_rel = tile_residues(a, g0), g0_lo = (uint32_t)g0;
     const uint32_t w_first = (warp * SQ_ROWS * 32 + lane) * 4;
-    if (w_first < nres_rel) {
-        const uint64_t g = g0 + w_first;
-        uint32_t lo = p_lo, hi = p_hi;
-        while (lo < hi) {
-            const uint32_t mid = (lo + hi + 1) >> 1;
-            if (offs[mid] <= g) lo = mid; else hi = mid - 1;
-        }
-        p = lo;
-        pstart_lo = (uint32_t)offs[p];
-        pend_rel = rel(offs[p + 1]);
-    }
+    uint32_t p = p_lo, pstart_lo = 0, pend_rel = 0;
+    if (w_first < nres_rel) first_protein(offs, g0, p_lo, p_hi, w_first, p, pstart_lo, pend_rel);
 
-    const uint32_t lt = (1u << lane) - 1u;
-    const uint32_t g0_lo = (uint32_t)g0;
     bool zero_seen = false;
     uint32_t wcount = 0;  // tuples staged by this warp so far (uniform across the warp)
-    // unordered output (SCATTER: the first level of the partition follows in this kernel): hashes stay in registers, a
-    // window's loc waits in its own staging slot -- no ranking of the kept windows
-    constexpr bool DIRECT = SCATTER && KS_DIRECT_SCATTER;
-    static_assert(DS_ITEMS == SQ_ROWS * 4, "a thread's windows are its scatter items");
-    uint64_t dkey[DIRECT ? DS_ITEMS : 1];
+    uint64_t dkey[SCATTER ? DS_ITEMS : 1];
     uint32_t dvalid = 0;
 #pragma unroll
     for (int rr = 0; rr < SQ_ROWS; rr++) {
         const uint32_t q = (warp * SQ_ROWS + rr) * 32 + lane;
-        uint32_t x[NW + 1];
-#pragma unroll
-        for (int i = 0; i < NW; i++) x[i] = s_res[q + i];
-        x[NW] = 0;
+        const Quad<K> quad(s_res, q);
         uint64_t h[4], loc[4];
         bool keep[4];
         // a quad that lies inside one protein with all four windows complete (9 in 10) skips the per-window walk
@@ -485,14 +526,10 @@ sketch_quad_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint
             const uint32_t w = q * 4 + j;
             bool valid = inside;
             if (!inside && w < nres_rel) {
-                while (w >= pend_rel) { p++; pstart_lo = (uint32_t)offs[p]; pend_rel = rel(offs[p + 1]); }
+                seek_protein(offs, g0, w, p, pstart_lo, pend_rel);
                 valid = w + K <= pend_rel;
             }
-            uint32_t b[KW];
-#pragma unroll
-            for (int i = 0; i < KW; i++) b[i] = j == 0 ? x[i] : __funnelshift_r(x[i], x[i + 1], 8 * j);
-            if (K % 4) b[KW - 1] &= (1u << (8 * (K % 4))) - 1u;
-            h[j] = murmur_limbs<K>(b);
+            h[j] = quad.hash(j);
             if (FULL) {
                 keep[j] = valid;  // the count was fixed in advance; a zero hash (1 in 2^64) sends the batch to the general path
                 zero_seen |= valid && h[j] == 0;
@@ -505,133 +542,58 @@ sketch_quad_kernel(SketchArgs a, Lut256 lut, uint32_t* __restrict__ ticket, uint
             }
             loc[j] = ((uint64_t)(a.pid_base + p) << 32) | (uint64_t)(g0_lo + w - pstart_lo);
         }
-        if (DIRECT) {
+        if (SCATTER) {
 #pragma unroll
             for (int j = 0; j < 4; j++) {
-                dkey[DIRECT ? rr * 4 + j : 0] = h[j];
+                dkey[SCATTER ? rr * 4 + j : 0] = h[j];
                 dvalid |= (keep[j] ? 1u : 0u) << (rr * 4 + j);
                 s_loc[(rr * 4 + j) * SK_THREADS + tid] = loc[j];
             }
-            continue;
-        }
-        uint32_t below = 0, total = 0;
-        uint32_t bal[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            bal[j] = __ballot_sync(0xffffffffu, keep[j]);
-            below += __popc(bal[j] & lt);
-            total += __popc(bal[j]);
-        }
-        uint32_t slot = warp * (SK_TILE / (SK_THREADS / 32)) + wcount + below;
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            if (keep[j]) {
-                const uint32_t ad = stage_addr(slot);
+        } else {
+            stage_row(lane, warp, keep, wcount, [&](int j, uint32_t ad) {
                 s_hash[ad] = h[j];
                 s_loc[ad] = loc[j];
-                slot++;
-            }
+            });
         }
-        wcount += total;
     }
 
     if (FULL && zero_seen) atomicOr(reinterpret_cast<uint32_t*>(a.d_count + 1) + 1, 1u);
-    if (DIRECT) {
-        static_assert(DS_THREADS == SK_THREADS && DS_TILE == SK_TILE, "one scatter tile per sketch tile");
+    if (SCATTER) {
         static_assert(OFFS_CACHE == SK_THREADS, "one protein counter per thread");
         __shared__ DenseScatterSmem s_sc;
         const uint32_t total = scatter_pairs(reinterpret_cast<const uint64_t (&)[DS_ITEMS]>(dkey), dvalid,
                                              [&](int it) { return s_loc[it * SK_THREADS + tid]; }, a.scatter, 0, s_sc, s_hash, s_loc);
-        if (COUNT_ABUND && cached && tid < n_off - 1) {  // (the scatter's barriers ordered the counts before this read)
+        if (COUNT_ABUND && cached && tid < p_hi - p_lo + 1) {  // (the scatter's barriers ordered the counts before this read)
             const uint32_t c = s_pcnt[tid];
             if (c) atomicAdd(&a.t_abund[p_lo + tid], c);
         }
         if (tid == 0 && total) atomicAdd(reinterpret_cast<unsigned long long*>(a.d_count), (unsigned long long)total);
         return;
     }
-    if (lane == 0) s_wtot[warp] = wcount;
-    __syncthreads();
-    uint32_t wprefix = 0, btotal = 0;
-#pragma unroll
-    for (int i = 0; i < SK_THREADS / 32; i++) {
-        const uint32_t t = s_wtot[i];
-        if (i < (int)warp) wprefix += t;
-        btotal += t;
-    }
-    if (SCATTER) {
-        // unordered output: the tile's tuples go straight into the first-level regions of the partition -- no tile base,
-        // and on the look-back path no look-back either (the total is all that is left to collect)
-        static_assert(DS_THREADS == SK_THREADS && DS_TILE == SK_TILE, "one scatter tile per sketch tile");
-        static_assert(OFFS_CACHE == SK_THREADS, "one protein counter per thread");
-        __shared__ DenseScatterSmem s_sc;
-        if (COUNT_ABUND && cached && tid < n_off - 1) {  // (the barrier after s_wtot ordered the counts before this read)
-            const uint32_t c = s_pcnt[tid];
-            if (c) atomicAdd(&a.t_abund[p_lo + tid], c);
-        }
-        if (tid == 0) {
-            if (btotal) atomicAdd(reinterpret_cast<unsigned long long*>(a.d_count), (unsigned long long)btotal);
-        }
-        uint64_t key[DS_ITEMS];
-        uint32_t valid = 0;
-#pragma unroll
-        for (int it = 0; it < DS_ITEMS; it++) {
-            const uint32_t i = it * SK_THREADS + tid;  // slot: warp region i >> 8, offset i & 255
-            key[it] = s_hash[stage_addr(i)];
-            valid |= ((i & 255u) < s_wtot[i >> 8] ? 1u : 0u) << it;
-        }
-        scatter_pairs(key, valid, [&](int it) { return s_loc[stage_addr(it * SK_THREADS + tid)]; }, a.scatter, 0, s_sc, s_hash, s_loc);
-        return;
-    }
-    uint64_t base;
-    if (FULL) {
-        base = tile_base[tile] + wprefix;
-        if (tid == 0 && tile == n_tiles - 1) *a.d_count = tile_base[tile] + btotal;
-    } else {
-        if (warp == 0) {
-            const uint64_t excl = scan_lookback(status, tile, btotal);
-            if (lane == 0) {
-                s_base = excl;
-                if (tile == n_tiles - 1) *a.d_count = excl + btotal;
-            }
-        }
-        __syncthreads();
-        base = s_base + wprefix;
-    }
-    const uint32_t sbase = warp * (SK_TILE / (SK_THREADS / 32));
-    if (base + wcount <= a.capacity) {  // the usual case: the warp's 256 slots, 8 per lane, no per-element bound check
-        uint64_t* oh = a.out_hash + base;
-        uint64_t* ol = a.out_loc + base;
-#pragma unroll
-        for (uint32_t i0 = 0; i0 < SK_TILE / (SK_THREADS / 32); i0 += 32) {
-            const uint32_t i = i0 + lane;
-            if (i0 >= wcount) break;  // uniform
-            if (i < wcount) {
-                const uint32_t ad = stage_addr(sbase + i);
-                oh[i] = s_hash[ad];
-                ol[i] = s_loc[ad];
-            }
-        }
-    } else {
-        for (uint32_t i = lane; i < wcount; i += 32) {
-            if (base + i < a.capacity) {
-                const uint32_t ad = stage_addr(sbase + i);
-                a.out_hash[base + i] = s_hash[ad];
-                a.out_loc[base + i] = s_loc[ad];
-            }
-        }
-    }
+    const WarpPrefix wp = warp_prefix(tid, s_wtot, wcount);
+    const uint64_t base = wp.wprefix + (FULL ? exact_base(tid, a, tile, tile_base, wp.btotal)
+                                             : lookback_base(lane, warp, a, tile, status, wp.btotal, s_base));
+    const uint32_t sbase = warp * WARP_SLOTS;
+    uint64_t* oh = a.out_hash + base;
+    uint64_t* ol = a.out_loc + base;
+    write_warp(lane, a, base, wcount, [&](uint32_t i) {
+        const uint32_t ad = stage_addr(sbase + i);
+        oh[i] = s_hash[ad];
+        ol[i] = s_loc[ad];
+    });
 }
 
 // ---------------------------------------------------------------------------------------------
-// Dense k-mer space (two-letter hp alphabet, K <= 24, scaled == 1): a window is a K-bit pattern and its hash a
-// function of the pattern, so the index is built from ranks instead of hashes.  `rank_of_code[pattern]` (a
-// per-handle table: all 2^K patterns hashed and sorted once, dense.cu) is the position of the pattern's hash among
-// all patterns' hashes; a tuple becomes ONE 64-bit key  rank | protein | position , the library sorts the keys on
-// the rank bits alone (stable, three passes of 8-byte keys for K = 24), and equal ranks ARE equal hashes: no bucket
-// sort, no second look at the hash.  This kernel is the exact-path sketch kernel with the hash replaced by a table
-// read: residues are staged and translated once per tile, turned into two bit streams (hydrophobic / neither
-// class), and a window's pattern is one funnel shift.  A complete window that holds a residue of neither class
-// (X, U, O, *) has no pattern: the kernel flags it and the host builds this batch on the general path.
+// Dense k-mer space (two-letter hp alphabet, K <= 24, scaled == 1; DESIGN.md 3.3): a window is a K-bit pattern, its hash
+// a function of the pattern, and its tuple ONE 64-bit key  code | protein | position.  `code_of_pattern` (a per-handle
+// table, dense.cu) gives every pattern an order-preserving code: the top DENSE_PREFIX_BITS bits of its hash, then its rank
+// among the patterns of that hash prefix (sketch.cuh), so keys sort like (hash, protein, position) tuples.  This is the
+// exact-path sketch kernel with the hash replaced by a table read: residues are staged and translated once per tile,
+// turned into two bit streams (hydrophobic / neither class), and a window's pattern is one funnel shift.  A complete
+// window that holds a residue of neither class (X, U, O, *) has no pattern: with handle_exceptions it is hashed from its
+// bytes and placed among the patterns' hashes (an even code); without, the kernel flags it and the host builds the batch
+// on the general path.  The keys leave either through the first level of the key sort (d.scatter.out != nullptr) or in
+// tile order at the tiles' exact bases (d.out_keys, sorted by the library afterwards).
 // ---------------------------------------------------------------------------------------------
 // 5 CTAs per SM: measured 2.41 ms (4), 1.78 ms (5), 1.89 ms (6, 40 registers) on C2
 #ifndef KS_DK_CTAS
@@ -654,58 +616,13 @@ sketch_dense_kernel(SketchArgs a, Lut256 lut, const uint32_t* __restrict__ tile_
 
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     s_lut[tid] = lut.b[tid];
-    if (tid < 32) {
-        const uint32_t c = tid;
-        s_lut32[c] = c == 0 ? 0 : c <= 26 ? lut.b['A' + c - 1] : c == 27 ? lut.b['*'] : 0;
-    }
+    if (tid < 32) s_lut32[tid] = lut32_entry(lut.b, tid);
     __syncthreads();
     const uint32_t tile = blockIdx.x + a.tile_begin;
     const uint64_t g0 = (uint64_t)tile * SK_TILE;
-    const uint64_t n_tiles = n_tiles_of(a.n_res);
     const uint32_t p_lo = tile_pid[tile], p_hi = tile_pid[tile + 1];
-    const uint32_t n_off = p_hi - p_lo + 2;
-    const bool cached = n_off <= OFFS_CACHE;
-    if (cached)
-        for (uint32_t i = tid; i < n_off; i += SK_THREADS) s_offs[i] = a.offsets[p_lo + i];
-    if (a.packed) {
-        constexpr uint32_t n_groups = (SK_TILE + K - 1 + 7) / 8;
-        for (uint32_t grp = tid; grp < n_groups; grp += SK_THREADS) {
-            const uint64_t group = g0 / 8 + grp;
-            const uint64_t byte = group * 5;
-            uint32_t w0 = 0, w1 = 0;
-            if (group * 8 < a.n_res) {  // groups past the last residue are not backed by memory
-                const uint32_t* w = reinterpret_cast<const uint32_t*>(a.residues + (byte & ~3ull));
-                w0 = __ldg(w);
-                w1 = __ldg(w + 1);
-            }
-            const uint32_t sh8 = (uint32_t)(byte & 3) * 8;
-            const uint32_t lo = __funnelshift_r(w0, w1, sh8), hi = (w1 >> sh8) & 0xffu;  // 40 bits: lo | hi << 32
-            uint32_t o0 = 0, o1 = 0;
-#pragma unroll
-            for (int i = 0; i < 4; i++) o0 |= (uint32_t)s_lut32[(lo >> (5 * i)) & 31u] << (8 * i);
-            o1 |= (uint32_t)s_lut32[(lo >> 20) & 31u];
-            o1 |= (uint32_t)s_lut32[(lo >> 25) & 31u] << 8;
-            o1 |= (uint32_t)s_lut32[((lo >> 30) | (hi << 2)) & 31u] << 16;
-            o1 |= (uint32_t)s_lut32[(hi >> 3) & 31u] << 24;
-            s_res[2 * grp] = o0;
-            s_res[2 * grp + 1] = o1;
-        }
-    } else {
-        constexpr uint32_t n_chunks = (SK_TILE + K - 1 + 15) / 16;
-        if (tid < n_chunks) {
-            const uint64_t g = g0 + 16ull * tid;
-            uint4 v = make_uint4(0, 0, 0, 0);
-            if (g < a.n_res) v = __ldg(reinterpret_cast<const uint4*>(a.residues + g));
-            uint32_t w[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-            for (int i = 0; i < 4; i++) {
-                const uint32_t x = w[i];
-                w[i] = (uint32_t)s_lut[x & 0xff] | ((uint32_t)s_lut[(x >> 8) & 0xff] << 8) |
-                       ((uint32_t)s_lut[(x >> 16) & 0xff] << 16) | ((uint32_t)s_lut[x >> 24] << 24);
-            }
-            reinterpret_cast<uint4*>(s_res)[tid] = make_uint4(w[0], w[1], w[2], w[3]);
-        }
-    }
+    const bool cached = cache_offsets(tid, a, s_offs, p_lo, p_hi);
+    stage_residues<true>(tid, s_res, a, a.packed, g0, SK_TILE + K - 1, s_lut, s_lut32);
     __syncthreads();
     // bit streams over the staged residues: bit i of word w = residue 32 w + i is hydrophobic / of neither class
     for (uint32_t wd = tid; wd < (uint32_t)N_BITW; wd += SK_THREADS) {
@@ -727,36 +644,16 @@ sketch_dense_kernel(SketchArgs a, Lut256 lut, const uint32_t* __restrict__ tile_
     __syncthreads();
 
     const uint64_t* offs = cached ? (const uint64_t*)s_offs - p_lo : a.offsets;
-    const uint64_t left = a.n_res - g0;
-    const uint32_t nres_rel = left > 0x40000000ull ? 0x40000000u : (uint32_t)left;  // residues from the tile start on
-    auto rel = [&](uint64_t o) -> uint32_t {  // protein end, relative to the tile start, clamped
-        const uint64_t dd = o - g0;
-        return dd > 0x7fffffffull ? 0x7fffffffu : (uint32_t)dd;
-    };
-    uint32_t p = p_lo, pstart_lo = 0, pend_rel = 0;
+    const uint32_t nres_rel = tile_residues(a, g0), g0_lo = (uint32_t)g0;
     const uint32_t w_first = (warp * SQ_ROWS * 32 + lane) * 4;
-    if (w_first < nres_rel) {
-        const uint64_t g = g0 + w_first;
-        uint32_t lo = p_lo, hi = p_hi;
-        while (lo < hi) {
-            const uint32_t mid = (lo + hi + 1) >> 1;
-            if (offs[mid] <= g) lo = mid; else hi = mid - 1;
-        }
-        p = lo;
-        pstart_lo = (uint32_t)offs[p];
-        pend_rel = rel(offs[p + 1]);
-    }
+    uint32_t p = p_lo, pstart_lo = 0, pend_rel = 0;
+    if (w_first < nres_rel) first_protein(offs, g0, p_lo, p_hi, w_first, p, pstart_lo, pend_rel);
 
     constexpr uint32_t KMASK = K >= 32 ? 0xffffffffu : ((1u << (K & 31)) - 1u);
-    const uint32_t lt = (1u << lane) - 1u;
-    const uint32_t g0_lo = (uint32_t)g0;
     const int loc_bits = d.pid_bits + d.pos_bits;
     bool exc_seen = false, exc_emitted = false;
     uint32_t wcount = 0;  // keys staged by this warp so far (uniform across the warp)
-    // unordered output (the first level of the key sort follows in this kernel): the keys stay in registers and go straight
-    // into the scatter -- no ranking of the kept windows, no staging in window order
-    static_assert(DS_ITEMS == SQ_ROWS * 4, "a thread's windows are its scatter items");
-    const bool direct = KS_DIRECT_SCATTER && d.scatter.out != nullptr;
+    const bool scatter = d.scatter.out != nullptr;
     uint64_t dkey[DS_ITEMS];
     uint32_t dvalid = 0;
 #pragma unroll
@@ -773,7 +670,7 @@ sketch_dense_kernel(SketchArgs a, Lut256 lut, const uint32_t* __restrict__ tile_
             const uint32_t w = q * 4 + j;
             bool valid = inside;
             if (!inside && w < nres_rel) {
-                while (w >= pend_rel) { p++; pstart_lo = (uint32_t)offs[p]; pend_rel = rel(offs[p + 1]); }
+                seek_protein(offs, g0, w, p, pstart_lo, pend_rel);
                 valid = w + K <= pend_rel;
             }
             const uint32_t bsh = ((q & 7u) << 2) + j;  // bit offset of window w in its stream word: (4q + j) mod 32
@@ -788,155 +685,62 @@ sketch_dense_kernel(SketchArgs a, Lut256 lut, const uint32_t* __restrict__ tile_
         for (int j = 0; j < 4; j++) {
             if (is_exc[j]) {  // rare: hash the translated bytes, place the hash among the patterns' hashes
                 if (!d.handle_exceptions) { exc_seen = true; continue; }
-                constexpr int NW = (K + 3 + 3) / 4, KW = (K + 3) / 4;
-                uint32_t x[NW + 1], bw[KW];
-#pragma unroll
-                for (int i = 0; i < NW; i++) x[i] = s_res[q + i];
-                x[NW] = 0;
-#pragma unroll
-                for (int i = 0; i < KW; i++) bw[i] = j == 0 ? x[i] : __funnelshift_r(x[i], x[i + 1], 8 * j);
-                if (K % 4) bw[KW - 1] &= (1u << (8 * (K % 4))) - 1u;
-                const uint64_t h = murmur_limbs<K>(bw);
+                const uint64_t h = Quad<K>(s_res, q).hash(j);
                 const uint32_t pfx = (uint32_t)(h >> (64 - DENSE_PREFIX_BITS));
-                const uint32_t g0 = __ldg(d.group_base + pfx), g1 = __ldg(d.group_base + pfx + 1);
-                uint32_t lo = g0, hi = g1;  // first pattern hash >= h inside the prefix group
+                const uint32_t gb0 = __ldg(d.group_base + pfx), gb1 = __ldg(d.group_base + pfx + 1);
+                uint32_t lo = gb0, hi = gb1;  // first pattern hash >= h inside the prefix group
                 while (lo < hi) {
                     const uint32_t mid = (lo + hi) >> 1;
                     if (__ldg(d.sorted_hash + mid) < h) lo = mid + 1; else hi = mid;
                 }
-                const bool same = lo < g1 && __ldg(d.sorted_hash + lo) == h;  // a pattern with this very hash
-                rank[j] = (pfx << d.rb) | (2u * (lo - g0) + (same ? 1u : 0u));
+                const bool same = lo < gb1 && __ldg(d.sorted_hash + lo) == h;  // a pattern with this very hash
+                rank[j] = (pfx << d.rb) | (2u * (lo - gb0) + (same ? 1u : 0u));
                 if (h == 0) exc_seen = true;  // would have to be dropped: general path
                 exc_emitted = true;
             }
         }
-        if (direct) {
+        if (scatter) {
 #pragma unroll
             for (int j = 0; j < 4; j++) {
                 dkey[rr * 4 + j] = ((uint64_t)rank[j] << loc_bits) | locp[j];
                 dvalid |= (keep[j] ? 1u : 0u) << (rr * 4 + j);
             }
-            continue;
+        } else {
+            stage_row(lane, warp, keep, wcount, [&](int j, uint32_t ad) { s_key[ad] = ((uint64_t)rank[j] << loc_bits) | locp[j]; });
         }
-        uint32_t below = 0, total = 0;
-        uint32_t bal[4];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            bal[j] = __ballot_sync(0xffffffffu, keep[j]);
-            below += __popc(bal[j] & lt);
-            total += __popc(bal[j]);
-        }
-        uint32_t slot = warp * (SK_TILE / (SK_THREADS / 32)) + wcount + below;
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            if (keep[j]) {
-                s_key[stage_addr(slot)] = ((uint64_t)rank[j] << loc_bits) | locp[j];
-                slot++;
-            }
-        }
-        wcount += total;
     }
     if (exc_seen) atomicOr(d.exception_flag, 1u);
     if (exc_emitted) atomicOr(d.exception_flag + 1, 1u);
-    __shared__ DenseScatterSmem s_sc;
-    if (direct) {
+    if (scatter) {
+        __shared__ DenseScatterSmem s_sc;
         const uint32_t total = scatter_keys(dkey, dvalid, d.scatter, 0, s_sc, s_key);
         if (tid == 0 && total) atomicAdd(reinterpret_cast<unsigned long long*>(a.d_count), (unsigned long long)total);
         return;
     }
-    if (lane == 0) s_wtot[warp] = wcount;
-    __syncthreads();
-    uint32_t wprefix = 0, btotal = 0;
-#pragma unroll
-    for (int i = 0; i < SK_THREADS / 32; i++) {
-        const uint32_t t = s_wtot[i];
-        if (i < (int)warp) wprefix += t;
-        btotal += t;
-    }
-    if (d.scatter.out != nullptr) {  // first level of the key sort, straight out of shared memory (no tile bases: unordered)
-        if (tid == 0 && btotal) atomicAdd(reinterpret_cast<unsigned long long*>(a.d_count), (unsigned long long)btotal);
-        static_assert(DS_THREADS == SK_THREADS && DS_TILE == SK_TILE, "one scatter tile per sketch tile");
-        uint64_t key[DS_ITEMS];
-        uint32_t valid = 0;
-#pragma unroll
-        for (int it = 0; it < DS_ITEMS; it++) {
-            const uint32_t i = it * SK_THREADS + tid;  // slot: warp region i >> 8, offset i & 255
-            key[it] = s_key[stage_addr(i)];
-            valid |= ((i & 255u) < s_wtot[i >> 8] ? 1u : 0u) << it;
-        }
-        scatter_keys(key, valid, d.scatter, 0, s_sc, s_key);  // the staging buffer is free once the keys are in registers
-        return;
-    }
-    const uint64_t base = tile_base[tile] + wprefix;
-    if (tid == 0 && tile == n_tiles - 1) *a.d_count = tile_base[tile] + btotal;
-    const uint32_t sbase = warp * (SK_TILE / (SK_THREADS / 32));
+    const WarpPrefix wp = warp_prefix(tid, s_wtot, wcount);
+    const uint64_t base = exact_base(tid, a, tile, tile_base, wp.btotal) + wp.wprefix;
+    const uint32_t sbase = warp * WARP_SLOTS;
     uint64_t* ok = d.out_keys + base;
 #pragma unroll
-    for (uint32_t i0 = 0; i0 < SK_TILE / (SK_THREADS / 32); i0 += 32) {
+    for (uint32_t i0 = 0; i0 < WARP_SLOTS; i0 += 32) {  // (one checked pass: write_warp's unrolled copy costs C2's scatter path 3 %)
         const uint32_t i = i0 + lane;
         if (i0 >= wcount) break;  // uniform
         if (i < wcount && base + i < a.capacity) ok[i] = s_key[stage_addr(sbase + i)];
     }
 }
 
-template <int K>
-struct DenseDispatch {
-    static cudaError_t run(const SketchArgs& a, const Lut256& lut, const Workspace& w, unsigned grid, const DenseSketchArgs& d,
-                           cudaStream_t st) {
-        if (a.k == (uint32_t)K) {
-            sketch_dense_kernel<K><<<grid, SK_THREADS, 0, st>>>(a, lut, w.tile_pid, w.tile_base, d);
-            return cudaGetLastError();
-        }
-        return DenseDispatch<K - 1>::run(a, lut, w, grid, d, st);
-    }
-};
-template <>
-struct DenseDispatch<DENSE_MIN_K - 1> {
-    static cudaError_t run(const SketchArgs&, const Lut256&, const Workspace&, unsigned, const DenseSketchArgs&, cudaStream_t) {
-        return cudaErrorInvalidValue;
-    }
-};
-
-template <int K>
-cudaError_t launch_k(const SketchArgs& a, const Lut256& lut, const Workspace& w, uint64_t n_tiles, cudaStream_t st) {
-    const bool ranged = a.tile_end > a.tile_begin;  // a sub-range of the tiles (the look-back path takes them by ticket:
-                                                    // ranges must be launched in order, each exactly once)
-    const unsigned grid = ranged ? (unsigned)(a.tile_end - a.tile_begin) : (unsigned)n_tiles;
-    if constexpr (K == 0) {
-        if (a.moltype == 0)
-            sketch_kernel<0, false><<<grid, SK_THREADS, 0, st>>>(a, lut, w.ticket, w.status, w.tile_pid);
-        else
-            sketch_kernel<0, true><<<grid, SK_THREADS, 0, st>>>(a, lut, w.ticket, w.status, w.tile_pid);
-    } else {
-        const bool full = a.max_hash == ~0ull && !a.force_general;
-        const bool sc = a.scatter.out_key != nullptr;
-#define KS_LAUNCH_QUAD(T, F, S) \
-    sketch_quad_kernel<K, T, F, S><<<grid, SK_THREADS, 0, st>>>(a, lut, w.ticket, w.status, w.tile_pid, w.tile_base)
-        if (a.moltype == 0) {
-            if (full) { if (sc) KS_LAUNCH_QUAD(false, true, true); else KS_LAUNCH_QUAD(false, true, false); }
-            else { if (sc) KS_LAUNCH_QUAD(false, false, true); else KS_LAUNCH_QUAD(false, false, false); }
-        } else {
-            if (full) { if (sc) KS_LAUNCH_QUAD(true, true, true); else KS_LAUNCH_QUAD(true, true, false); }
-            else { if (sc) KS_LAUNCH_QUAD(true, false, true); else KS_LAUNCH_QUAD(true, false, false); }
-        }
-#undef KS_LAUNCH_QUAD
-    }
-    return cudaGetLastError();
+// Calls f(std::integral_constant<int, V>()) for the run-time value v = V in [LO, HI]; cudaErrorInvalidValue outside.
+template <int LO, int HI, class F>
+cudaError_t dispatch(int v, F&& f) {
+    if constexpr (LO > HI) return cudaErrorInvalidValue;
+    else return v == HI ? f(std::integral_constant<int, HI>()) : dispatch<LO, HI - 1>(v, f);
 }
 
-template <int K>
-struct Dispatch {
-    static cudaError_t run(const SketchArgs& a, const Lut256& lut, const Workspace& w, uint64_t nt, cudaStream_t st) {
-        if (a.k == (uint32_t)K) return launch_k<K>(a, lut, w, nt, st);
-        return Dispatch<K - 1>::run(a, lut, w, nt, st);
-    }
-};
-template <>
-struct Dispatch<0> {
-    static cudaError_t run(const SketchArgs& a, const Lut256& lut, const Workspace& w, uint64_t nt, cudaStream_t st) {
-        return launch_k<0>(a, lut, w, nt, st);
-    }
-};
+// Tiles [a.tile_begin, a.tile_end) of the batch, or all tiles when the range is empty (the look-back path takes tiles by
+// ticket: its ranges must be launched in order, each exactly once).
+unsigned grid_of(const SketchArgs& a, uint64_t n_tiles) {
+    return a.tile_end > a.tile_begin ? (unsigned)(a.tile_end - a.tile_begin) : (unsigned)n_tiles;
+}
 
 }  // namespace
 
@@ -1025,16 +829,31 @@ cudaError_t launch_sketch_prepare(const SketchArgs& a, cudaStream_t stream, uint
     return cudaSuccess;
 }
 
-// The fused kernel over tiles [a.tile_begin, a.tile_end) (exact path; 0, 0 = all tiles).
+// The sketch kernel over tiles [a.tile_begin, a.tile_end) (0, 0 = all tiles).
 cudaError_t launch_sketch_tiles(const SketchArgs& a, cudaStream_t stream, uint64_t* n_launches) {
     if (a.n_res == 0 || a.n_prot == 0) return cudaSuccess;
-    const uint64_t nt = n_tiles_of(a.n_res);
-    Workspace w = carve(a.workspace, a.n_res);
+    const Workspace w = carve(a.workspace, a.n_res);
+    const unsigned grid = grid_of(a, n_tiles_of(a.n_res));
     Lut256 lut;
     fill_lut(a.moltype, &lut);
-    cudaError_t e = Dispatch<SK_MAX_TEMPLATE_K>::run(a, lut, w, nt, stream);
     if (n_launches) *n_launches += 1;
-    return e;
+    if (a.k > (uint32_t)SK_MAX_TEMPLATE_K) {
+        if (a.moltype == 0) sketch_kernel<false><<<grid, SK_THREADS, 0, stream>>>(a, lut, w.ticket, w.status, w.tile_pid);
+        else sketch_kernel<true><<<grid, SK_THREADS, 0, stream>>>(a, lut, w.ticket, w.status, w.tile_pid);
+        return cudaGetLastError();
+    }
+    const bool translate = a.moltype != 0, full = exact_path(a), scatter = a.scatter.out_key != nullptr;
+    return dispatch<1, SK_MAX_TEMPLATE_K>((int)a.k, [&](auto K) {
+        return dispatch<0, 1>(translate, [&](auto T) {
+            return dispatch<0, 1>(full, [&](auto F) {
+                return dispatch<0, 1>(scatter, [&](auto S) {
+                    sketch_quad_kernel<K, T != 0, F != 0, S != 0>
+                        <<<grid, SK_THREADS, 0, stream>>>(a, lut, w.ticket, w.status, w.tile_pid, w.tile_base);
+                    return cudaGetLastError();
+                });
+            });
+        });
+    });
 }
 
 // Look-back path: d_count[1] <- 0 (no zero-hash flag there: such a hash fails h != 0 and is dropped in the kernel).  The
@@ -1057,14 +876,15 @@ cudaError_t launch_sketch(const SketchArgs& a, cudaStream_t stream, uint64_t* n_
 cudaError_t launch_sketch_dense(const SketchArgs& a, const DenseSketchArgs& d, cudaStream_t stream, uint64_t* n_launches) {
     if (a.n_res == 0 || a.n_prot == 0) return cudaSuccess;
     if (a.moltype != 2 || a.k < (uint32_t)DENSE_MIN_K || a.k > (uint32_t)DENSE_MAX_K || a.max_hash != ~0ull) return cudaErrorInvalidValue;
-    const uint64_t nt = n_tiles_of(a.n_res);
-    Workspace w = carve(a.workspace, a.n_res);
+    const Workspace w = carve(a.workspace, a.n_res);
+    const unsigned grid = grid_of(a, n_tiles_of(a.n_res));
     Lut256 lut;
     fill_lut(a.moltype, &lut);
-    const bool ranged = a.tile_end > a.tile_begin;
-    const unsigned grid = ranged ? (unsigned)(a.tile_end - a.tile_begin) : (unsigned)nt;
     if (n_launches) *n_launches += 1;
-    return DenseDispatch<DENSE_MAX_K>::run(a, lut, w, grid, d, stream);
+    return dispatch<DENSE_MIN_K, DENSE_MAX_K>((int)a.k, [&](auto K) {
+        sketch_dense_kernel<K><<<grid, SK_THREADS, 0, stream>>>(a, lut, w.tile_pid, w.tile_base, d);
+        return cudaGetLastError();
+    });
 }
 
 }  // namespace ks

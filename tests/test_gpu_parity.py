@@ -791,22 +791,31 @@ def test_pipelined_upload_matches_single_copy(K, monkeypatch, k, moltype, scaled
         assert np.array_equal(a, b)
 
 
-def test_unpackable_residues_take_the_byte_path(K, O):
+def test_unpackable_residues_take_the_byte_path(K, O, monkeypatch):
     """Index builds upload 5-bit packed residues; a proteome handed over with bytes outside A-Z and '*'
-    (ks_proteome_from_packed does not validate) cannot be packed and must go through the plain byte path."""
+    (ks_proteome_from_packed does not validate) cannot be packed and must go through the plain byte path, on every
+    route of the sketch kernels: the ordered sketch, the dense path with its own key sort (every hp window of these bytes
+    has a residue of neither class: exception keys) and with the library's (no exception handling: general path), and,
+    on a batch large enough for the unstable partition, the sketch kernel's scatter at scaled 1 and at scaled > 1.  The
+    large batch has a run of 1 000 proteins of 0-3 residues, more than the sketch kernel's offsets cache holds for one
+    tile, so that kept windows are counted per protein both in shared memory and in global memory."""
     rng = np.random.default_rng(8)
-    res = rng.choice(np.frombuffer(b"ACDEFGHIKLMNPQRSTVWYacdxyz@#1", dtype=np.uint8), size=50_000)
+    alphabet = np.frombuffer(b"ACDEFGHIKLMNPQRSTVWYacdxyz@#1", dtype=np.uint8)
+    res = rng.choice(alphabet, size=50_000)
     offs = np.array([0, 10_000, 10_000, 35_000, 50_000], dtype=np.uint64)
-    prot = K.Proteome.from_packed(res, offs)
-    for k, moltype in ((7, "protein"), (12, "hp")):
-        with K.ProteomeIndex("db", k, 1, moltype) as idx:
-            idx.add_proteome(prot)
-            idx.finalize()
-            keys, row_ptr, pid, pos = idx.csr()
-            oh, opid, opos = O.sketch_tuples(res, offs, k, moltype, 1)
-            okeys, orow, ops, oqs = O.build_index(oh, opid, opos)
-            assert np.array_equal(keys, okeys) and np.array_equal(row_ptr, orow)
-            assert np.array_equal(pid, ops) and np.array_equal(pos, oqs)
+    lens = np.concatenate([np.full(100, 3000), rng.integers(0, 4, size=1000), np.full(166, 3000)])
+    big_offs = np.concatenate([[0], np.cumsum(lens)]).astype(np.uint64)
+    big_res = rng.choice(alphabet, size=int(big_offs[-1]))
+    # (residues, offsets, k, moltype, scaled, KS_DENSE_SORT, build_path): 0 general (ordered sketch), 1 dense with the
+    # hand-written key sort, 3 general with the unstable partition
+    cases = [(res, offs, 7, "protein", 1, None, 0), (res, offs, 12, "hp", 1, None, 1), (res, offs, 12, "hp", 1, "library", 0),
+             (big_res, big_offs, 7, "protein", 1, None, 3), (big_res, big_offs, 7, "protein", 10, None, 3)]
+    for r, o, k, moltype, scaled, dense_sort, path in cases:
+        if dense_sort:
+            monkeypatch.setenv("KS_DENSE_SORT", dense_sort)
+        else:
+            monkeypatch.delenv("KS_DENSE_SORT", raising=False)
+        _csr_equals_oracle(K, O, r, o, k, moltype, scaled=scaled, path=path)
 
 
 def test_golden_zstd_fasta(K, golden_rust):
