@@ -152,7 +152,10 @@ ks_status ks_index_sync(ks_index *idx);
  *              = the end state of combined_minhash / signatures after process_fasta (:907-961).
  * ks_index_add_proteome = upload + sketch (residues streamed in chunks, hashed as they land).  ks_index_clear drops
  * tuples and the CSR and keeps the resident batch: clear + ks_index_sketch_resident + ks_index_finalize builds it again
- * (the benchmark loop).  A build costs ONE host read-back (counts and flags, at the end of finalize).  */
+ * (the benchmark loop).  A build costs ONE host read-back (counts and flags, at the end of finalize).
+ * A finalized index takes no more adds; ks_index_append_* extends it instead: the batch is built on its own by the same
+ * stages and merged into the index on the device (one pass over the old postings, no rebuild, the old residues are not
+ * needed), and the index is finalized again on return.  */
 ks_status ks_index_upload(ks_index *idx, const ks_proteome *p);
 ks_status ks_index_sketch_resident(ks_index *idx);
 ks_status ks_index_add_proteome(ks_index *idx, const ks_proteome *p);
@@ -164,6 +167,17 @@ ks_status ks_index_process_fasta(ks_index *idx, const char *path, uint64_t ambig
  * tuples with protein ids local to the batch (0..n_proteins-1). */
 ks_status ks_index_add_tuples(ks_index *idx, const uint64_t *hash, const uint32_t *pid, const uint32_t *pos,
                               uint64_t n, uint64_t n_proteins);
+/* Extend a FINALIZED index by one batch; the index is finalized again on return.  The batch's proteins get the ids
+ * n_proteins .. n_proteins + batch - 1.  The result is the index that add(old batches) + add(batch) + finalize gives
+ * (CSR, export, combined sketch, signature_count, search); stats count the merged totals and build_path is 4.
+ * = a repeated process_fasta (src/rust/index.rs:907-961) on the same index.  Not finalized: KS_ERR_NOT_FINALIZED;
+ * more than 2^31-1 tuples or 2^32-2 proteins in the merged index: KS_ERR_CAPACITY.  A failed append leaves the index as
+ * it was.  The appended batch becomes the resident batch.  Device memory while appending: about twice the index.
+ * An appended index cannot take part in ks_shard_search_batch (KS_ERR_VALIDATION). */
+ks_status ks_index_append_proteome(ks_index *idx, const ks_proteome *p);
+/* store_signatures (src/rust/index.rs:800-830) on a finalized index: arguments as ks_index_add_tuples. */
+ks_status ks_index_append_tuples(ks_index *idx, const uint64_t *hash, const uint32_t *pid, const uint32_t *pos,
+                                 uint64_t n, uint64_t n_proteins);
 
 typedef struct ks_stats {
     uint64_t n_proteins;      /* proteins added (signatures incl. ones whose id collides) */
@@ -185,7 +199,8 @@ typedef struct ks_stats {
     uint32_t build_path;     /* how the last finalize built the index: 0 general (hash tuples, partition + bucket sort),
                                 1 dense k-mer space (hp, 8 <= k <= 24, scaled 1: rank keys), 2 the same with the keys
                                 sorted by the library, 3 general with the unstable two-level partition (one batch of
-                                hashes that rarely repeat) */
+                                hashes that rarely repeat), 4 a finalized index extended by ks_index_append_*, compact
+                                layout */
 } ks_stats;
 /* Synchronises the handle's stream. */
 ks_status ks_index_stats(ks_index *idx, ks_stats *out);

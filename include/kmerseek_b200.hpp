@@ -141,6 +141,25 @@ class ProteomeIndex {
         }
         check(ks_index_add_tuples(h_, h.data(), pid.data(), pos.data(), h.size(), sigs.size()));
     }
+    // store_signatures on a finalized index: the signatures are merged into it (ks_index_append_tuples)
+    void append_signatures(const std::vector<ProteinSignature>& sigs) {
+        std::vector<uint64_t> h;
+        std::vector<uint32_t> pid, pos;
+        for (size_t i = 0; i < sigs.size(); i++) {
+            h.insert(h.end(), sigs[i].hashes.begin(), sigs[i].hashes.end());
+            pos.insert(pos.end(), sigs[i].positions.begin(), sigs[i].positions.end());
+            pid.insert(pid.end(), sigs[i].hashes.size(), (uint32_t)i);
+        }
+        check(ks_index_append_tuples(h_, h.data(), pid.data(), pos.data(), h.size(), sigs.size()));
+    }
+    // a repeated process_fasta on a finalized index: read, then merge the batch in (ks_index_append_proteome)
+    void append_fasta(const std::string& fasta_path) {
+        ks_proteome* p = nullptr;
+        check(ks_proteome_from_fasta(fasta_path.c_str(), 0, &p));
+        const ks_status st = ks_index_append_proteome(h_, p);
+        ks_proteome_free(p);
+        check(st);
+    }
     // process_fasta (src/rust/index.rs:907-961); progress_interval / batch_size kept for signature parity
     void process_fasta(const std::string& fasta_path, uint32_t /*progress_interval*/ = 0, size_t /*batch_size*/ = 1000) {
         check(ks_index_process_fasta(h_, fasta_path.c_str(), 0));

@@ -102,6 +102,8 @@ SIGNATURES = {
     "ks_index_clear": (C.c_int, [C.c_void_p]),
     "ks_index_process_fasta": (C.c_int, [C.c_void_p, C.c_char_p, C.c_uint64]),
     "ks_index_add_tuples": (C.c_int, [C.c_void_p, u64p, u32p, u32p, C.c_uint64, C.c_uint64]),
+    "ks_index_append_proteome": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "ks_index_append_tuples": (C.c_int, [C.c_void_p, u64p, u32p, u32p, C.c_uint64, C.c_uint64]),
     "ks_index_stats": (C.c_int, [C.c_void_p, C.POINTER(ks_stats)]),
     "ks_index_signature_count": (C.c_int, [C.c_void_p, u64p]),
     "ks_sketch_batch": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(C.POINTER(ks_sketch))]),

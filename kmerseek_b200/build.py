@@ -7,7 +7,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OUT = os.path.join(HERE, "libkmerseek_b200.so")
-SOURCES = ["api.cu", "sketch.cu", "index_build.cu", "dense.cu", "search.cu"]
+SOURCES = ["api.cu", "sketch.cu", "index_build.cu", "dense.cu", "search.cu", "append.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 EXTRA = os.environ.get("KS_NVCC_EXTRA", "").split()  # experiments: -DKS_...=...
 FLAGS = EXTRA + ["-std=c++17", "-O3", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo",

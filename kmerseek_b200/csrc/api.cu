@@ -12,6 +12,7 @@
 
 #include <nccl.h>  // types and prototypes only: the library is bound with dlopen (NcclApi), never linked
 
+#include "append.cuh"
 #include "dense.cuh"
 #include "host_util.hpp"
 #include "ingest.hpp"
@@ -459,8 +460,16 @@ struct Csr {
     uint32_t seg_nb = 0;
     const uint32_t* seg_start = nullptr;
     const uint64_t* seg_counts = nullptr;
+    uint64_t* hash = nullptr;  // sorted tuples: the hash column (see hash_col_valid) and the postings
+    uint64_t* loc = nullptr;
     uint64_t U = 0, G = 0, n_ids = 0;
-    bool hash_col_valid = true;  // false: d_hash of the sorted tuples is rebuilt on demand (ks_index_export)
+    bool hash_col_valid = true;  // false: the sorted hash column is rebuilt on demand (ks_index_export)
+};
+
+// Buffers of a finalized index of its own: where an index extended by ks_index_append_* lives (two sets, ping-pong: the
+// next append merges from one into the other, and a build never touches either).
+struct CsrSet {
+    Buf keys, key_grp, grp_start, t_size, t_abund, dir, hash, loc, seg_start, seg_counts;
 };
 
 // The device words a build reports through (ks_index::d_status), one block so that they are zeroed and read back together.
@@ -484,6 +493,8 @@ struct Hooks {
     bool timing = false;          // KS_TIMING: host-side stage timings on stderr
     bool search_legacy = false;   // KS_SEARCH_LEGACY: the library-sorted query path for every batch
     int ls_variant = 0;           // KS_LS_VARIANT = rep | bn | bs: bucket-sort variant of the stable path (1 / 2 / 3)
+    int append_fail = 0;          // KS_APPEND_FAIL = build | merge: an append fails as an allocation would, after the
+                                  // batch's build (1) or after the merge kernels (2), to test that the index is restored
     void read() {
         sketch_general = getenv("KS_SKETCH_GENERAL") != nullptr;
         const char* d = getenv("KS_DENSE");
@@ -497,6 +508,8 @@ struct Hooks {
         search_legacy = getenv("KS_SEARCH_LEGACY") != nullptr;
         const char* lv = getenv("KS_LS_VARIANT");
         ls_variant = !lv ? 0 : lv[0] == 'r' ? 1 : (lv[0] == 'b' && lv[1] == 's') ? 3 : lv[0] == 'b' ? 2 : 0;
+        const char* af = getenv("KS_APPEND_FAIL");
+        append_fail = !af ? 0 : af[0] == 'b' ? 1 : af[0] == 'm' ? 2 : 0;
     }
 };
 
@@ -508,7 +521,7 @@ struct ks_index {
     cudaStream_t stream = nullptr;
     cudaStream_t copy_stream = nullptr;  // H2D of residue chunks while earlier tiles are being hashed
     cudaEvent_t ev_chunk[17] = {};
-    cudaEvent_t ev[12] = {};
+    cudaEvent_t ev[13] = {};
     uint64_t live_bytes = 0;
     Arena* arena = nullptr;
 
@@ -542,6 +555,12 @@ struct ks_index {
     int dense_pid_bits = 0, dense_pos_bits = 0;
     Csr csr;
     Buf b_keys, b_key_grp, b_grp_start, b_t_size, b_t_abund, b_dir, b_alt_hash, b_alt_loc, b_temp;
+    // append: the index lives in the build's buffers (home -1) or in app[home]; scratch of the merge (compact copies of
+    // segmented inputs, the per-key insertion points)
+    CsrSet app[2];
+    int home = -1;
+    bool appended = false;  // the index holds batches merged by ks_index_append_* (no sharded search)
+    Buf b_ca_keys, b_ca_kg, b_ca_gs, b_ca_dir, b_cb_keys, b_cb_kg, b_cb_gs, b_m_pre, b_m_counts, b_m_work;
     // query path: per-handle scratch (grow-only) and a pinned word block for the counts the host reads back
     Buf b_q_ecount, b_q_pcount, b_q_hcount, b_q_sig, b_q_poff, b_q_hoff, b_q_ent_hash, b_q_ent_abund, b_q_win_key,
         b_q_win_hoff, b_q_stage, b_q_totals;
@@ -558,7 +577,7 @@ struct ks_index {
 
 namespace {
 
-enum { EV_UP0, EV_UP1, EV_SK0, EV_SK1, EV_SO0, EV_SO1, EV_CS0, EV_CS1, EV_Q0, EV_Q1, EV_PART };
+enum { EV_UP0, EV_UP1, EV_SK0, EV_SK1, EV_SO0, EV_SO1, EV_CS0, EV_CS1, EV_Q0, EV_Q1, EV_PART, EV_M0, EV_M1 };
 // pinned words of a handle: [0, QT_WORDS) totals of the query kernels; then this rank's header of a sharded search;
 // then every rank's header
 enum { HW_TOTALS = 0, HW_HDR = QT_WORDS, HW_ALL = QT_WORDS + 8, H_WORDS = QT_WORDS + 8 + 4 * MAX_SHARDS };
@@ -594,6 +613,8 @@ void upload_batch(ks_index* x, DeviceBatch& b, const ks_proteome* p, bool allow_
 void drop_content(ks_index* x) {
     x->state = Build::Tuples;
     x->csr = Csr();
+    x->home = -1;
+    x->appended = false;
     x->n_tuples = x->n_prot = x->n_res = x->n_windows = 0;
 }
 
@@ -994,12 +1015,16 @@ void dense_rank_tiles(ks_index* x, uint32_t t0, uint32_t t1) {
 // The CSR's buffers for n tuples of P proteins.  The directory has about 4 tuples (<= 4 keys) per bucket, so that it stays
 // small next to the keys, and at least the 2^top_bits buckets of the key sort (a directory bucket must not span two of
 // them); the key, group and directory arrays get `slack` more slots.
-Csr reserve_csr(ks_index* x, uint64_t n, uint32_t P, int top_bits, uint64_t slack) {
+int dir_bits_for(uint64_t n) {
     int bits = 8;
     while (bits < 24 && (4ull << bits) < n) bits++;
+    return bits;
+}
+
+Csr reserve_csr(ks_index* x, uint64_t n, uint32_t P, int top_bits, uint64_t slack) {
     Arena* ar = x->arena;
     Csr c;
-    c.dir_bits = std::max(bits, top_bits);
+    c.dir_bits = std::max(dir_bits_for(n), top_bits);
     c.dir_shift = 64 - x->lz - c.dir_bits;
     c.t_abund = x->b_t_abund.ensure<uint32_t>(ar, P);
     c.t_size = x->b_t_size.ensure<uint32_t>(ar, P);
@@ -1069,6 +1094,7 @@ bool dense_finalize(ks_index* x) {
     if ((uint32_t)st.overflow) return false;  // heavy repeats of one k-mer overflowed a sort bucket: the general path handles those
     cs.U = st.U; cs.G = st.G;
     cs.hash_col_valid = false;  // d_hash holds code keys: the sorted hash column is rebuilt from the CSR on demand
+    cs.hash = x->d_hash; cs.loc = x->d_loc;
     x->csr = cs;
     x->build_path = plan.custom ? 1u : 2u;
     x->state = Build::Finalized;
@@ -1145,6 +1171,7 @@ void finalize(ks_index* x) {
     }
     cs.U = st.U; cs.G = st.G;
     cs.hash_col_valid = hash_written != 0;
+    cs.hash = x->d_hash; cs.loc = x->d_loc;
     x->csr = cs;
     x->build_path = scattered ? 3u : 0u;
     x->state = Build::Finalized;
@@ -1154,11 +1181,218 @@ void finalize(ks_index* x) {
 CsrView view_of(const ks_index* x) {
     const Csr& c = x->csr;
     CsrView v;
-    v.hash = x->d_hash; v.loc = x->d_loc; v.keys = c.keys; v.key_grp = c.key_grp; v.grp_start = c.grp_start;
+    v.hash = c.hash; v.loc = c.loc; v.keys = c.keys; v.key_grp = c.key_grp; v.grp_start = c.grp_start;
     v.t_size = c.t_size; v.t_abund = c.t_abund; v.dir = c.dir; v.d_counts = c.d_counts; v.n = x->n_tuples;
     v.n_prot = (uint32_t)x->n_prot; v.dir_bits = c.dir_bits; v.dir_shift = c.dir_shift;
     v.dir_sub = c.dir_sub; v.seg_nb = c.seg_nb; v.seg_start = c.seg_start; v.seg_counts = c.seg_counts;
     return v;
+}
+
+// The resident batch replaced by p (ks_index_upload).
+void upload_resident(ks_index* x, const ks_proteome* p) {
+    materialize_pending(x);  // the resident batch is about to be replaced
+    KS_CUDA(cudaEventRecord(x->ev[EV_UP0], x->stream));
+    upload_batch(x, x->batch, p, true);
+    KS_CUDA(cudaEventRecord(x->ev[EV_UP1], x->stream));
+    x->t_upload = true;
+}
+
+// ks_index_add_proteome: the pipelined add, or upload + sketch of the resident batch.
+void add_proteome(ks_index* x, const ks_proteome* p) {
+    if (add_proteome_pipelined(x, p)) return;
+    upload_resident(x, p);
+    sketch_resident(x);
+}
+
+// The postings of host tuples with protein ids local to their batch (+ pid_base); checks range and (protein, pos) order.
+std::vector<uint64_t> tuple_locs(const uint32_t* pid, const uint32_t* pos, uint64_t n, uint64_t n_proteins, uint32_t pid_base) {
+    std::vector<uint64_t> loc(n);
+    for (uint64_t i = 0; i < n; i++) {
+        if (pid[i] >= n_proteins) fail(KS_ERR_VALIDATION, "Validation error: tuple protein index out of range");
+        loc[i] = ((uint64_t)(pid[i] + pid_base) << 32) | pos[i];
+        if (i && loc[i] <= loc[i - 1]) fail(KS_ERR_VALIDATION, "Validation error: tuples must be ordered by (protein, pos)");
+    }
+    return loc;
+}
+
+// Tuples behind the ones the (not finalized) handle holds, n_proteins more proteins.
+void push_tuples(ks_index* x, const uint64_t* hash, const std::vector<uint64_t>& loc, uint64_t n_proteins) {
+    const uint64_t n = loc.size();
+    grow_tuples(x, x->n_tuples + n);
+    if (n) {
+        KS_CUDA(cudaMemcpyAsync(x->d_hash + x->n_tuples, hash, n * 8, cudaMemcpyHostToDevice, x->stream));
+        KS_CUDA(cudaMemcpyAsync(x->d_loc + x->n_tuples, loc.data(), n * 8, cudaMemcpyHostToDevice, x->stream));
+        KS_CUDA(cudaStreamSynchronize(x->stream));
+    }
+    x->n_tuples += n;
+    x->n_prot += n_proteins;
+}
+
+// ---- append (ks_index_append_*) -----------------------------------------------------------------------------------------
+// The finalized index A is parked, the batch is built as the handle's only content by the usual routes (B), and the two
+// are merged into a compact index C in the append set A does not occupy.  A failure anywhere puts A back as it was.
+struct Parked {
+    Csr csr;
+    uint64_t n_tuples = 0, n_prot = 0, n_res = 0, n_windows = 0;
+    uint32_t build_path = 0;
+    int home = -1;
+    bool appended = false;
+};
+
+// An index in the build's buffers moves to app[0]: its buffers are swapped with the set's (no copy), the tuple pair too;
+// the segmented layout's bucket tables live in the build's scratch and are copied.  An index in an append set stays.
+// Everything that can fail (the tables' allocations and copies) comes first: the swaps that follow cannot, so the index
+// is either where it was or wholly in app[0] with home = 0.
+void park_index(ks_index* x) {
+    if (x->home >= 0) return;
+    CsrSet& s = x->app[0];
+    Csr& c = x->csr;
+    const uint32_t* seg_start = c.seg_start;
+    const uint64_t* seg_counts = c.seg_counts;
+    if (c.dir_sub != DIR_SUB_COMPACT) {
+        uint32_t* st = s.seg_start.ensure<uint32_t>(x->arena, (uint64_t)c.seg_nb + 1);
+        uint64_t* sc = s.seg_counts.ensure<uint64_t>(x->arena, c.seg_nb);
+        KS_CUDA(cudaMemcpyAsync(st, c.seg_start, ((uint64_t)c.seg_nb + 1) * 4, cudaMemcpyDeviceToDevice, x->stream));
+        KS_CUDA(cudaMemcpyAsync(sc, c.seg_counts, (uint64_t)c.seg_nb * 8, cudaMemcpyDeviceToDevice, x->stream));
+        seg_start = st; seg_counts = sc;
+    }
+    std::swap(x->b_keys, s.keys); std::swap(x->b_key_grp, s.key_grp); std::swap(x->b_grp_start, s.grp_start);
+    std::swap(x->b_t_size, s.t_size); std::swap(x->b_t_abund, s.t_abund); std::swap(x->b_dir, s.dir);
+    Buf h{x->d_hash, x->cap * 8}, l{x->d_loc, x->cap * 8};
+    std::swap(h, s.hash); std::swap(l, s.loc);
+    if (h.p && l.p) {  // the set's former pair becomes the build's tuple pair
+        x->d_hash = (uint64_t*)h.p; x->d_loc = (uint64_t*)l.p; x->cap = std::min(h.bytes, l.bytes) / 8;
+    } else {
+        if (h.p) x->arena->release(h.p);
+        if (l.p) x->arena->release(l.p);
+        x->d_hash = x->d_loc = nullptr; x->cap = 0;
+    }
+    c.seg_start = seg_start; c.seg_counts = seg_counts;
+    x->home = 0;
+}
+
+void restore_index(ks_index* x, const Parked& a) {
+    x->csr = a.csr;
+    x->n_tuples = a.n_tuples; x->n_prot = a.n_prot; x->n_res = a.n_res; x->n_windows = a.n_windows;
+    x->build_path = a.build_path; x->home = a.home; x->appended = a.appended;
+    x->state = Build::Finalized;
+    try {  // the batch's build has overwritten the totals the device reads (d_counts)
+        const uint64_t ug[2] = {a.csr.U, a.csr.G};
+        KS_CUDA(cudaMemcpyAsync(x->d_status, ug, 16, cudaMemcpyHostToDevice, x->stream));
+        KS_CUDA(cudaStreamSynchronize(x->stream));
+    } catch (...) {
+    }
+}
+
+// One input of the merge in the compact layout: a segmented index is compacted into scratch (keys, key_grp, grp_start).
+MergeSide merge_side(ks_index* x, const Csr& c, uint64_t n, Buf& bk, Buf& bkg, Buf& bgs, uint64_t* counts) {
+    MergeSide m;
+    m.U = c.U; m.G = c.G; m.n = n; m.loc = c.loc;
+    if (c.dir_sub == DIR_SUB_COMPACT) {
+        m.keys = c.keys; m.key_grp = c.key_grp; m.grp_start = c.grp_start;
+        return m;
+    }
+    Arena* ar = x->arena;
+    uint64_t* keys = bk.ensure<uint64_t>(ar, c.U);
+    uint32_t* kg = bkg.ensure<uint32_t>(ar, c.U + 1);
+    uint32_t* gs = bgs.ensure<uint32_t>(ar, c.G + 1);
+    uint32_t* pre = x->b_m_pre.ensure<uint32_t>(ar, 2ull * c.seg_nb);
+    CsrView v;
+    v.keys = c.keys; v.key_grp = c.key_grp; v.grp_start = c.grp_start; v.n = n;
+    v.seg_nb = c.seg_nb; v.seg_start = c.seg_start; v.seg_counts = c.seg_counts;
+    KS_CUDA(launch_compact_segmented(v, c.U, c.G, pre, keys, kg, gs, counts, x->stream, &x->l_csr));
+    m.keys = keys; m.key_grp = kg; m.grp_start = gs;
+    return m;
+}
+
+// A (parked) + B (the handle's finalized batch) -> C in the other append set.
+void merge_appended(ks_index* x, const Parked& A, double batch_ms) {
+    Arena* ar = x->arena;
+    const Csr B = x->csr;
+    const uint64_t n_b = x->n_tuples, p_b = x->n_prot;
+    const uint64_t n = A.n_tuples + n_b, P = A.n_prot + p_b, G = A.csr.G + B.G, U_max = A.csr.U + B.U;
+    if (n > MAX_TUPLES) fail(KS_ERR_CAPACITY, "more than 2^31-1 tuples on one shard: shard the proteome over more GPUs");
+    const int dst = 1 - A.home;
+    CsrSet& out = x->app[dst];
+    uint64_t* counts = x->b_m_counts.ensure<uint64_t>(ar, 4);
+    KS_CUDA(cudaEventRecord(x->ev[EV_M0], x->stream));
+    const MergeSide a = merge_side(x, A.csr, A.n_tuples, x->b_ca_keys, x->b_ca_kg, x->b_ca_gs, counts);
+    const MergeSide b = merge_side(x, B, n_b, x->b_cb_keys, x->b_cb_kg, x->b_cb_gs, counts + 2);
+    const uint32_t* dir_a = A.csr.dir;
+    if (A.csr.dir_sub != DIR_SUB_COMPACT) {  // a directory over the compacted keys (same bits)
+        uint32_t* d = x->b_ca_dir.ensure<uint32_t>(ar, (1ull << A.csr.dir_bits) + 1);
+        KS_CUDA(launch_directory(a.keys, counts, d, A.csr.dir_bits, A.csr.dir_shift, x->stream));
+        x->l_csr += 1;
+        dir_a = d;
+    }
+    Csr c;
+    c.dir_bits = dir_bits_for(n);
+    c.dir_shift = 64 - x->lz - c.dir_bits;
+    c.keys = out.keys.ensure<uint64_t>(ar, U_max);
+    c.key_grp = out.key_grp.ensure<uint32_t>(ar, U_max + 1);
+    c.grp_start = out.grp_start.ensure<uint32_t>(ar, G + 1);
+    c.t_size = out.t_size.ensure<uint32_t>(ar, P);
+    c.t_abund = out.t_abund.ensure<uint32_t>(ar, P);
+    c.dir = out.dir.ensure<uint32_t>(ar, (1ull << c.dir_bits) + 2);
+    c.hash = out.hash.ensure<uint64_t>(ar, n);
+    c.loc = out.loc.ensure<uint64_t>(ar, n);
+    c.d_counts = x->d_status;
+    AppendArgs m;
+    m.a = a; m.b = b; m.dir_a = dir_a; m.dir_bits_a = A.csr.dir_bits; m.dir_shift_a = A.csr.dir_shift; m.p_a = (uint32_t)A.n_prot;
+    m.keys = c.keys; m.key_grp = c.key_grp; m.grp_start = c.grp_start; m.loc = c.loc; m.d_counts = x->d_status;
+    m.work_bytes = append_work_bytes(B.U);
+    m.work = x->b_m_work.ensure<char>(ar, m.work_bytes);
+    KS_CUDA(launch_append_merge(m, x->stream, &x->l_csr));
+    KS_CUDA(launch_directory(c.keys, x->d_status, c.dir, c.dir_bits, c.dir_shift, x->stream));
+    x->l_csr += 1;
+    if (A.n_prot) {
+        KS_CUDA(cudaMemcpyAsync(c.t_size, A.csr.t_size, A.n_prot * 4, cudaMemcpyDeviceToDevice, x->stream));
+        KS_CUDA(cudaMemcpyAsync(c.t_abund, A.csr.t_abund, A.n_prot * 4, cudaMemcpyDeviceToDevice, x->stream));
+    }
+    if (p_b) {
+        KS_CUDA(cudaMemcpyAsync(c.t_size + A.n_prot, B.t_size, p_b * 4, cudaMemcpyDeviceToDevice, x->stream));
+        KS_CUDA(cudaMemcpyAsync(c.t_abund + A.n_prot, B.t_abund, p_b * 4, cudaMemcpyDeviceToDevice, x->stream));
+    }
+    KS_CUDA(cudaEventRecord(x->ev[EV_M1], x->stream));
+    const StatusBlock st = read_status(x, StatusBlock{}, 24);  // U_C, G_C, M: the one host read of the merge
+    if (st.G != G || st.U + st.produced != U_max) fail(KS_ERR_CUDA, "internal error: the merged index does not add up");
+    if (x->hooks.append_fail == 2) fail(KS_ERR_OUT_OF_MEMORY, "KS_APPEND_FAIL: append failed after the merge (test hook)");
+    c.U = st.U; c.G = st.G;
+    c.hash_col_valid = false;  // rebuilt from the CSR on demand (ks_index_export)
+    if (x->hooks.timing) {
+        float ms = 0;
+        KS_CUDA(cudaEventElapsedTime(&ms, x->ev[EV_M0], x->ev[EV_M1]));
+        fprintf(stderr, "[ks] append: batch_path %u A_layout %s B_layout %s U_A %llu U_B %llu matched %llu n_C %llu batch_ms %.3f merge_ms %.3f\n",
+                x->build_path, A.csr.dir_sub == DIR_SUB_COMPACT ? "compact" : "seg", B.dir_sub == DIR_SUB_COMPACT ? "compact" : "seg",
+                (unsigned long long)A.csr.U, (unsigned long long)B.U, (unsigned long long)st.produced, (unsigned long long)n,
+                batch_ms, ms);
+    }
+    x->csr = c;
+    x->n_tuples = n; x->n_prot = P; x->n_res += A.n_res; x->n_windows += A.n_windows;
+    x->build_path = 4;
+    x->home = dst;
+    x->appended = true;
+}
+
+// Extend the finalized index by the batch add_batch() adds.
+template <class F>
+void append_batch(ks_index* x, F&& add_batch) {
+    const double t0 = wall_ms();
+    park_index(x);
+    Parked A;
+    A.csr = x->csr; A.n_tuples = x->n_tuples; A.n_prot = x->n_prot; A.n_res = x->n_res; A.n_windows = x->n_windows;
+    A.build_path = x->build_path; A.home = x->home; A.appended = x->appended;
+    try {
+        drop_content(x);
+        add_batch();
+        finalize(x);
+        if (x->hooks.append_fail == 1) fail(KS_ERR_OUT_OF_MEMORY, "KS_APPEND_FAIL: append failed after the batch's build (test hook)");
+        if (x->hooks.timing) KS_CUDA(cudaStreamSynchronize(x->stream));
+        merge_appended(x, A, wall_ms() - t0);
+    } catch (...) {
+        restore_index(x, A);
+        throw;
+    }
 }
 
 template <class T>
@@ -1274,26 +1508,18 @@ ks_status ks_index_upload(ks_index* x, const ks_proteome* p) {
     return guarded([&] {
         if (!x || !p) fail(KS_ERR_VALIDATION, "Validation error: null argument");
         x->use();
-        materialize_pending(x);  // the resident batch is about to be replaced
-        KS_CUDA(cudaEventRecord(x->ev[EV_UP0], x->stream));
-        upload_batch(x, x->batch, p, true);
-        KS_CUDA(cudaEventRecord(x->ev[EV_UP1], x->stream));
-        x->t_upload = true;
+        upload_resident(x, p);
     });
 }
 ks_status ks_index_sketch_resident(ks_index* x) {
     return guarded([&] { x->use(); sketch_resident(x); });
 }
 ks_status ks_index_add_proteome(ks_index* x, const ks_proteome* p) {
-    bool done = false;
-    ks_status s = guarded([&] {
+    return guarded([&] {
         if (!x || !p) fail(KS_ERR_VALIDATION, "Validation error: null argument");
         x->use();
-        done = add_proteome_pipelined(x, p);
+        add_proteome(x, p);
     });
-    if (s != KS_OK || done) return s;
-    s = ks_index_upload(x, p);
-    return s != KS_OK ? s : ks_index_sketch_resident(x);
 }
 ks_status ks_index_finalize(ks_index* x) {
     return guarded([&] { x->use(); finalize(x); });
@@ -1320,21 +1546,36 @@ ks_status ks_index_add_tuples(ks_index* x, const uint64_t* hash, const uint32_t*
         x->use();
         materialize_pending(x);
         if (x->n_prot + n_proteins >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins on one shard");
-        std::vector<uint64_t> loc(n);
-        for (uint64_t i = 0; i < n; i++) {
-            if (pid[i] >= n_proteins) fail(KS_ERR_VALIDATION, "Validation error: tuple protein index out of range");
-            loc[i] = ((uint64_t)(pid[i] + (uint32_t)x->n_prot) << 32) | pos[i];
-            if (i && loc[i] <= loc[i - 1]) fail(KS_ERR_VALIDATION, "Validation error: tuples must be ordered by (protein, pos)");
-        }
+        const std::vector<uint64_t> loc = tuple_locs(pid, pos, n, n_proteins, (uint32_t)x->n_prot);
         if (x->finalized()) fail(KS_ERR_VALIDATION, "Validation error: index is finalized; ks_index_clear before adding more");
-        grow_tuples(x, x->n_tuples + n);
-        if (n) {
-            KS_CUDA(cudaMemcpyAsync(x->d_hash + x->n_tuples, hash, n * 8, cudaMemcpyHostToDevice, x->stream));
-            KS_CUDA(cudaMemcpyAsync(x->d_loc + x->n_tuples, loc.data(), n * 8, cudaMemcpyHostToDevice, x->stream));
-            KS_CUDA(cudaStreamSynchronize(x->stream));
-        }
-        x->n_tuples += n;
-        x->n_prot += n_proteins;
+        push_tuples(x, hash, loc, n_proteins);
+    });
+}
+
+ks_status ks_index_append_proteome(ks_index* x, const ks_proteome* p) {
+    return guarded([&] {
+        if (!x || !p) fail(KS_ERR_VALIDATION, "Validation error: null argument");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized: ks_index_finalize before appending");
+        x->use();
+        if (x->n_prot + p->n_prot >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins on one shard");
+        uint64_t windows = 0, max_len = 0;
+        proteome_shape(p, x->params.ksize, &windows, &max_len);
+        if (x->max_hash == ~0ull && x->n_tuples + windows > MAX_TUPLES)  // scaled 1: every window is a tuple
+            fail(KS_ERR_CAPACITY, "more than 2^31-1 tuples on one shard: shard the proteome over more GPUs");
+        append_batch(x, [&] { add_proteome(x, p); });
+    });
+}
+
+ks_status ks_index_append_tuples(ks_index* x, const uint64_t* hash, const uint32_t* pid, const uint32_t* pos, uint64_t n,
+                                 uint64_t n_proteins) {
+    return guarded([&] {
+        if (!x || (n && (!hash || !pid || !pos))) fail(KS_ERR_VALIDATION, "Validation error: null argument");
+        if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized: ks_index_finalize before appending");
+        x->use();
+        if (x->n_prot + n_proteins >= 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-2 proteins on one shard");
+        if (x->n_tuples + n > MAX_TUPLES) fail(KS_ERR_CAPACITY, "more than 2^31-1 tuples on one shard: shard the proteome over more GPUs");
+        const std::vector<uint64_t> loc = tuple_locs(pid, pos, n, n_proteins, 0);  // the batch's own ids: it is built alone
+        append_batch(x, [&] { push_tuples(x, hash, loc, n_proteins); });
     });
 }
 
@@ -1421,11 +1662,11 @@ ks_status ks_index_export(ks_index* x, ks_sketch** out) {
         Arena keep(x->stream, &x->live_bytes), tmp(x->stream, &x->live_bytes);
         Grouped g;
         if (!x->csr.hash_col_valid) {
-            KS_CUDA(expand_sorted_hash(view_of(x), x->d_hash, x->stream));
+            KS_CUDA(expand_sorted_hash(view_of(x), x->csr.hash, x->stream));
             x->csr.hash_col_valid = true;
         }
-        group_by_owner(keep, tmp, x->d_hash, x->d_loc, x->n_tuples, (uint32_t)x->n_prot, x->end_bit(), &g, &x->l_csr);
-        *out = sketch_to_host(g, x->d_hash, x->d_loc, x->n_tuples, x->n_prot, x->stream);
+        group_by_owner(keep, tmp, x->csr.hash, x->csr.loc, x->n_tuples, (uint32_t)x->n_prot, x->end_bit(), &g, &x->l_csr);
+        *out = sketch_to_host(g, x->csr.hash, x->csr.loc, x->n_tuples, x->n_prot, x->stream);
     });
 }
 
@@ -1448,7 +1689,7 @@ ks_status ks_index_csr(ks_index* x, ks_csr** out) {
         uint64_t* keys = to_host(x->csr.keys, seg ? span : x->csr.U, x->stream);
         uint32_t* kg = to_host(x->csr.key_grp, span, x->stream);
         uint32_t* gs = to_host(x->csr.grp_start, seg ? span : x->csr.G + 1, x->stream);
-        uint64_t* loc = to_host(x->d_loc, x->n_tuples, x->stream);
+        uint64_t* loc = to_host(x->csr.loc, x->n_tuples, x->stream);
         uint32_t* st = seg ? to_host(x->csr.seg_start, (uint64_t)x->csr.seg_nb + 1, x->stream) : nullptr;
         uint64_t* sc = seg ? to_host(x->csr.seg_counts, x->csr.seg_nb, x->stream) : nullptr;
         KS_CUDA(cudaStreamSynchronize(x->stream));
@@ -1789,6 +2030,9 @@ ks_status ks_shard_search_batch(ks_index* x, ks_comm* c, const ks_proteome* quer
     return guarded([&] {
         if (!c || !out) fail(KS_ERR_VALIDATION, "Validation error: null argument");
         if (!x->finalized()) fail(KS_ERR_NOT_FINALIZED, "index is not finalized");
+        if (x->appended)
+            fail(KS_ERR_VALIDATION, "Validation error: a sharded search needs an index built by adds and one finalize; this one was "
+                                    "extended by ks_index_append_* (rebuild it: ks_index_clear, add every batch, finalize)");
         if (c->device != x->params.device) fail(KS_ERR_VALIDATION, "Validation error: communicator and index are on different devices");
         if (pid_base + x->n_prot > 0xffffffffull) fail(KS_ERR_CAPACITY, "more than 2^32-1 proteins over all shards");
         x->use();

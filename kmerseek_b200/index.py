@@ -379,14 +379,22 @@ class ProteomeIndex:
         """src/rust/index.rs:800-830: add already-made signatures to the index."""
         if not protein_signatures:
             return
-        h = np.concatenate([s._hashes for s in protein_signatures]).astype(np.uint64)
-        pos = np.concatenate([s._positions for s in protein_signatures]).astype(np.uint32)
-        pid = np.concatenate([np.full(len(s._hashes), i, dtype=np.uint32) for i, s in enumerate(protein_signatures)])
+        h, pid, pos = self._signature_tuples(protein_signatures)
         check(_ffi.lib().ks_index_add_tuples(self._h, h.ctypes.data_as(_ffi.u64p), pid.ctypes.data_as(_ffi.u32p),
                                              pos.ctypes.data_as(_ffi.u32p), len(h), len(protein_signatures)))
         self._names.extend(s.name for s in protein_signatures)
         if self._store_raw:
             self._raw.extend(s._sequence for s in protein_signatures)
+
+    @staticmethod
+    def _signature_tuples(protein_signatures):
+        """(hash, protein, pos) of every kept window, protein ids local to the list."""
+        if not protein_signatures:
+            return np.zeros(0, np.uint64), np.zeros(0, np.uint32), np.zeros(0, np.uint32)
+        h = np.concatenate([s._hashes for s in protein_signatures]).astype(np.uint64)
+        pos = np.concatenate([s._positions for s in protein_signatures]).astype(np.uint32)
+        pid = np.concatenate([np.full(len(s._hashes), i, dtype=np.uint32) for i, s in enumerate(protein_signatures)])
+        return h, pid, pos
 
     def store_signatures_batch(self, protein_signatures):
         self.store_signatures(list(protein_signatures))
@@ -409,6 +417,31 @@ class ProteomeIndex:
         self.finalize()
         if progress_interval:
             print(f"Successfully processed and stored {n} sequences.")
+
+    def append_proteome(self, proteome: Proteome):
+        """Extend the finalized index by one batch (ks_index_append_proteome): the batch is built on the device and merged
+        into the index, which stays finalized; its proteins take the ids after the ones already there."""
+        check(_ffi.lib().ks_index_append_proteome(self._h, proteome._h))
+        self._names.extend(proteome.names)
+        if self._store_raw:
+            self._raw.extend(proteome.sequence(i) for i in range(proteome.n_proteins))
+
+    def append_fasta(self, fasta_path):
+        """A repeated process_fasta (src/rust/index.rs:907-961) on a finalized index: read, then append_proteome."""
+        prot = Proteome.from_fasta(fasta_path, self.ambig_seed)
+        try:
+            self.append_proteome(prot)
+        finally:
+            prot.close()
+
+    def append_signatures(self, protein_signatures):
+        """store_signatures (src/rust/index.rs:800-830) on a finalized index (ks_index_append_tuples)."""
+        h, pid, pos = self._signature_tuples(protein_signatures)
+        check(_ffi.lib().ks_index_append_tuples(self._h, h.ctypes.data_as(_ffi.u64p), pid.ctypes.data_as(_ffi.u32p),
+                                                pos.ctypes.data_as(_ffi.u32p), len(h), len(protein_signatures)))
+        self._names.extend(s.name for s in protein_signatures)
+        if self._store_raw:
+            self._raw.extend(s._sequence for s in protein_signatures)
 
     def finalize(self):
         check(_ffi.lib().ks_index_finalize(self._h))

@@ -83,6 +83,10 @@ extern "C" {
     pub fn ks_index_add_proteome(idx: *mut ks_index, p: *const ks_proteome) -> c_int;
     pub fn ks_index_finalize(idx: *mut ks_index) -> c_int;
     pub fn ks_index_process_fasta(idx: *mut ks_index, path: *const c_char, ambig_seed: u64) -> c_int;
+    // a repeated process_fasta / store_signatures (src/rust/index.rs:800-830, 907-961) on a finalized index
+    pub fn ks_index_append_proteome(idx: *mut ks_index, p: *const ks_proteome) -> c_int;
+    pub fn ks_index_append_tuples(idx: *mut ks_index, hash: *const u64, pid: *const u32, pos: *const u32, n: u64,
+                                  n_proteins: u64) -> c_int;
     pub fn ks_index_stats(idx: *mut ks_index, out: *mut ks_stats) -> c_int;
     pub fn ks_index_signature_count(idx: *mut ks_index, out: *mut u64) -> c_int; // src/rust/index.rs:514-516
     pub fn ks_sketch_batch(idx: *mut ks_index, p: *const ks_proteome, out: *mut *mut ks_sketch) -> c_int;
